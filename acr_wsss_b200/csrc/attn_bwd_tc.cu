@@ -13,7 +13,8 @@
 //               registers in one go and hands tS/tDP back at once (sdp_free), so the scores of tile i+1 run on the tensor
 //               pipe UNDER the exponentials of tile i; P and dS stay in registers until the gradient MMAs of tile i-1 have
 //               released the single-buffered smem tiles (pds_free)
-//   warps 12-15 drain: per tile dQ from TMEM -> fp32 staging tile -> two cp.reduce.async.bulk.tensor (fp32 add); per item
+//   warps 12-15 drain: per tile dQ from TMEM -> 64-bit fixed-point staging -> four cp.reduce.async.bulk.tensor (u64 add,
+//               order-independent, so the result is the same every run); per item
 //               dK / dV from TMEM -> bf16 rows of d_qkv
 // The softmax warps therefore execute nothing but the element-wise chain (round 1's kernel spent ~75 % of their time in
 // barrier waits, the dQ hand-over and the exposed S/dP MMA latency: profiles/r01g_ncu_attn_bwd_full.txt).
@@ -33,7 +34,7 @@ struct BwdSmem {
   uint8_t d_o[NST][TILE_BYTES];    // tile and the TMA refill takes ~1500 cycles (two stages left that latency exposed every tile)
   uint8_t p[2][TILE_BYTES];        // [kv block of 64][q row][64 kv] bf16, SWIZZLE_128B rows (one row per thread)
   uint8_t ds[2][TILE_BYTES];       // same layout: read MN-major (A = dS^T / P^T) and K-major (A = dS)
-  uint8_t dq[2][TILE_BYTES];       // fp32 staging of one dQ tile: [32-column half][q row][32 floats], SWIZZLE_128B
+  uint8_t dq[2][TILE_BYTES];       // dQ staging: two [q row][16 u64 fixed-point columns] boxes, SWIZZLE_128B (see drain_box)
   float stat[2][2][BM];            // [tile parity][0: lse * log2(e), 1: delta][q row]
   uint64_t kv_full, kv_empty, dkv_free, qdo_full[NST], qdo_empty[NST], stat_full[2], sdp_full, sdp_free, pds_full, pds_free, dq_full, dq_free;
   uint32_t tmem_base;
@@ -313,8 +314,8 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
 attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
                 const __grid_constant__ CUtensorMap tmap_dq,
                 const float* __restrict__ lse, const float* __restrict__ delta, const float* __restrict__ g_mean, long long g_bs,
-                long long g_ld, GCode gc, __nv_bfloat16* __restrict__ d_qkv, float* __restrict__ g_row0, int N, int H, int HB, float scale,
-                float scale_log2) {
+                long long g_ld, GCode gc, __nv_bfloat16* __restrict__ d_qkv, float* __restrict__ g_row0, int* __restrict__ dq_bad, float dq_lim,
+                int N, int H, int HB, float scale, float scale_log2) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   BwdSmem& s = *reinterpret_cast<BwdSmem*>(smem_raw);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -510,15 +511,43 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
       run([&](const SoftmaxArgs& sa, int T0) { bwd_softmax_loop<0, true>(s, sa, T0); }, true);
     }
   } else {
-    // drain warpgroup.  Per tile: dQ (rows = queries, 64 d columns) -> fp32 accumulator [B*H, N, 64] by two TMA reduce-adds of
-    // [128 x 32] fp32 SWIZZLE_128B tiles (rows past N are clipped by the tensor map).  Per item: dV, dK rows (lanes = keys) of
-    // the key tile -> d_qkv as bf16 once its last MMA has retired (the last dq_full of the item covers every earlier MMA).
+    // drain warpgroup.  Per tile: dQ (rows = queries, 64 d columns) -> 64-bit fixed-point accumulator [B*H, N, 64] (kDqFix) by
+    // four TMA reduce-adds of [128 x 16] u64 SWIZZLE_128B boxes, staged alternately in the two 16 KB halves of the staging buffer
+    // so that one box is staged while the other is read (rows past N are clipped by the tensor map).  Per item: dV, dK rows
+    // (lanes = keys) of the key tile -> d_qkv as bf16 once its last MMA has retired (the last dq_full of the item covers every
+    // earlier MMA).
     tc::reg_dealloc<REG_DRAIN>();
     const int row = (warp & 3) * 32 + lane;
     const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
     const bool leader = (warp == 12 && lane == 0);
     const uint32_t dq_row = (tc::smem_u32(s.dq[0]) + row * 128) ^ ((uint32_t)(row & 7) << 4);      // row start ^ swizzle term
     uint32_t r[32];
+    // one box: columns col .. col+15 of query tile i from r[base .. base+15] (fp32) through staging half `buf`.  The box staged
+    // there before is the older of the (at most) two in flight: wait until the TMA has read it.
+    auto drain_box = [&](int base, int buf, int col, int i, int hb) {
+      if (leader) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+      asm volatile("bar.sync 3, 128;" ::: "memory");
+      bool bad = false;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const float fa = __uint_as_float(r[base + 2 * e]) * kDqFix, fb = __uint_as_float(r[base + 2 * e + 1]) * kDqFix;
+        const bool oka = fabsf(fa) < dq_lim, okb = fabsf(fb) < dq_lim;          // false for NaN too
+        bad |= !(oka && okb);
+        const long long a = oka ? __float2ll_rn(fa) : 0ll, b = okb ? __float2ll_rn(fb) : 0ll;
+        sts128((dq_row + buf * TILE_BYTES) ^ (uint32_t)(e << 4), (uint32_t)a, (uint32_t)((unsigned long long)a >> 32), (uint32_t)b,
+               (uint32_t)((unsigned long long)b >> 32));
+      }
+      if (bad && i * BM + row < N) dq_bad[(size_t)hb * N + i * BM + row] = 1;        // the whole row of dQ comes out as NaN
+      tc::fence_proxy_async_smem();
+      asm volatile("bar.sync 3, 128;" ::: "memory");
+      if (leader) {
+        asm volatile("cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(
+                         reinterpret_cast<uint64_t>(&tmap_dq)),
+                     "r"(tc::smem_u32(s.dq[buf])), "r"(col), "r"(i * BM), "r"(hb)
+                     : "memory");
+        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+      }
+    };
     int T = 0, kvt, hb;
     bool tail;
     for (int k = 0; items.at(cta, G, k, kvt, hb, tail); ++k) {
@@ -527,33 +556,18 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_const
         tc::mbar_wait(&s.dq_full, T & 1);
         tc::tc_fence_after();
         if (warp == 12) BWD_TRACE(2, T, 1);
-        if (T > 0) {          // the reduce-add of the previous tile must have read the staging tile
-          if (leader) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-          asm volatile("bar.sync 3, 128;" ::: "memory");
-        }
-        if (warp == 12) BWD_TRACE(2, T, 2);
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          tc::tmem_ld32(tDQ + lane_off + c * 32, r);
-          tc::tmem_ld_wait();
-#pragma unroll
-          for (int e = 0; e < 8; ++e)
-            sts128((dq_row + c * TILE_BYTES) ^ (uint32_t)(e << 4), r[4 * e], r[4 * e + 1], r[4 * e + 2], r[4 * e + 3]);
-        }
+        tc::tmem_ld32(tDQ + lane_off, r);
+        tc::tmem_ld_wait();
+        drain_box(0, 0, 0, i, hb);
+        drain_box(16, 1, 16, i, hb);
+        tc::tmem_ld32(tDQ + lane_off + 32, r);
+        tc::tmem_ld_wait();
         tc::tc_fence_before();
-        tc::mbar_arrive(&s.dq_free);
-        tc::fence_proxy_async_smem();
-        asm volatile("bar.sync 3, 128;" ::: "memory");
-        if (leader) {
-#pragma unroll
-          for (int hh = 0; hh < 2; ++hh)
-            asm volatile("cp.reduce.async.bulk.tensor.3d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(
-                             reinterpret_cast<uint64_t>(&tmap_dq)),
-                         "r"(tc::smem_u32(s.dq[hh])), "r"(hh * 32), "r"(i * BM), "r"(hb)
-                         : "memory");
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-          BWD_TRACE(2, T, 3);
-        }
+        tc::mbar_arrive(&s.dq_free);                   // tDQ has been read
+        if (warp == 12) BWD_TRACE(2, T, 2);
+        drain_box(0, 0, 32, i, hb);
+        drain_box(16, 1, 48, i, hb);
+        if (leader) BWD_TRACE(2, T, 3);
       }
       // dV / dK of this item
       const int h = hb % H, b = hb / H, kv0 = kvt * BN;
@@ -600,7 +614,7 @@ namespace acr_attn {
 
 int launch_attn_bwd(const CUtensorMap& tmap_qkv, const CUtensorMap& tmap_do, const CUtensorMap& tmap_dq, const float* lse, const float* delta,
                     const float* g_mean, long long g_bs, long long g_ld, const GCode& gc, __nv_bfloat16* d_qkv, float* g_row0,
-                    int B, int N, int H, float scale, cudaStream_t st) {
+                    int* dq_bad, int B, int N, int H, float scale, cudaStream_t st) {
   const size_t smem = sizeof(BwdSmem);
   static bool attr_set[64] = {false};
   if (int e = set_max_smem(attn_bwd_kernel, smem, attr_set)) return e;
@@ -613,8 +627,8 @@ int launch_attn_bwd(const CUtensorMap& tmap_qkv, const CUtensorMap& tmap_do, con
   const long long nitems = (long long)kt * H * B;
   const unsigned grid = (unsigned)(nitems < sms[dev] ? nitems : sms[dev]);      // persistent: one CTA per SM
   acr::KernelTimer kt_("attn_bwd_kernel", st);
-  attn_bwd_kernel<<<grid, BWD_THREADS, smem, st>>>(tmap_qkv, tmap_do, tmap_dq, lse, delta, g_mean, g_bs, g_ld, gc, d_qkv, g_row0, N, H, H * B,
-                                                    scale, scale * kLog2e);
+  attn_bwd_kernel<<<grid, BWD_THREADS, smem, st>>>(tmap_qkv, tmap_do, tmap_dq, lse, delta, g_mean, g_bs, g_ld, gc, d_qkv, g_row0, dq_bad,
+                                                    dq_fix_limit(kt), N, H, H * B, scale, scale * kLog2e);
   return acr::check_launch("attn_bwd_kernel");
 }
 

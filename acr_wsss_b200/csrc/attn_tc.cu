@@ -291,8 +291,8 @@ struct MeanSmem {
 constexpr int STAGE_LD = 129;                  // fp32 staging row stride (conflict-free)
 static_assert(sizeof(float) * BM * STAGE_LD <= sizeof(uint8_t) * MEAN_STAGES * 2 * TILE_BYTES, "staging tile must fit");
 
-// MODE 0: mean[b,q,kv] = (1/H) sum_h P_h ; MODE 1 (backward pre-pass): delta[b,h,q] += (1/H) sum_kv P_h[q,kv] * G[b,q,kv]
-// (`mean` is then the read-only G, `p_row0` the delta accumulator).
+// MODE 0: mean[b,q,kv] = (1/H) sum_h P_h ; MODE 1 (backward pre-pass): part[kv tile][b,h,q] = (1/H) sum_kv P_h[q,kv] * G[b,q,kv]
+// over the CTA's key tile (`mean` is then the read-only G, `p_row0` the partial planes).
 // Softmax side: MEAN_SW warps = 4 TMEM lane quadrants x (MEAN_SW / 4) column slices of MEAN_COLS columns; each thread owns
 // one query row and MEAN_COLS key columns of the tile.  16 warps (4 per scheduler) instead of 8: the per-head chain
 // wait -> tcgen05.ld -> wait -> 32 exponentials of a warp is latency bound (clock64 timeline: 1500 cycles per head against
@@ -455,16 +455,18 @@ attn_mean_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const float* __re
       if (MODE == 1) s.part[slice][h][row] = part;
     }
     if (MODE == 1) {
-      // delta[b,h,q] += the four slices' sums: ONE atomic per (row, head) of the CTA, issued after the head loop (one per thread
-      // and head inside the loop was 4x the atomics -- 4.8 M per launch -- in the loop's way)
+      // this key tile's share of delta[b,h,q] (the four slices' sums) -> partial plane blockIdx.x, one store per (row, head) of the
+      // CTA after the head loop; bwd_delta_kernel adds the planes in key-tile order (a float atomic here would make the sum's
+      // rounding depend on which CTA lands first)
       asm volatile("bar.sync 1, %0;" ::"n"(MEAN_SW * 32) : "memory");
+      float* plane = p_row0 + (size_t)blockIdx.x * gridDim.z * H * N;
       for (int idx = sidx; idx < H * BM; idx += MEAN_SW * 32) {
         const int hh = idx / BM, rr = idx % BM;
         if (q0 + rr < N) {
           float v = 0.f;
 #pragma unroll
           for (int sl = 0; sl < MEAN_SW_SLICES; ++sl) v += s.part[sl][hh][rr];
-          atomicAdd(p_row0 + ((size_t)b * H + hh) * N + q0 + rr, v);
+          plane[((size_t)b * H + hh) * N + q0 + rr] = v;
         }
       }
     }
@@ -578,18 +580,20 @@ extern "C" int acr_attn_fwd_bf16(const void* qkv, int B, int N, int H, int D, fl
 // =============================================================================================
 // Backward.  dP_h = dO_h V_h^T + G/H ; dS_h = P_h * (dP_h - delta) ; delta[q] = sum_j P_h[q,j] dP_h[q,j]
 //   = dO_q . O_q + (1/H) sum_j P_h[q,j] G[q,j]   (the second term is what the affinity gradient adds).
-// Kernels: bwd_delta_kernel (dO.O, zero-fill of the dQ accumulator) -> attn_mean_kernel<1> (+ P.G/H) -> attn_bwd_kernel
-// (attn_bwd_tc.cu: persistent, rows = queries, dQ tiles reduced across kv tiles by TMA reduce-adds) -> bwd_dq_convert_kernel.
+// Kernels: attn_mean_kernel<1> (P.G/H per key tile) -> bwd_delta_kernel (dO.O + the key tiles' P.G/H in order, zero-fill of
+// the dQ accumulator) -> attn_bwd_kernel (attn_bwd_tc.cu: persistent, rows = queries, dQ tiles reduced across kv tiles by TMA
+// reduce-adds in 64-bit fixed point) -> bwd_dq_convert_kernel.  Every sum has a fixed order or is exact: same result every run.
 // =============================================================================================
 namespace {
 
 
 __global__ void __launch_bounds__(256)
-bwd_delta_kernel(const __nv_bfloat16* __restrict__ out, const __nv_bfloat16* __restrict__ d_out, float* __restrict__ delta,
-                 float4* __restrict__ dq_acc, long long rows, int N, int H) {
-  // delta[b,h,n] = dO[b,n,h,:] . O[b,n,h,:].  A warp takes 4 consecutive (b,n,h) rows at a time: 8 lanes x 16 bytes per 128-byte
-  // row (fully coalesced 512-byte requests), 3 shuffles.  The same pass zeroes the fp32 dQ accumulator the backward kernel
-  // reduces into (64 floats per row), which saves a separate memset node per block of the ViT.
+bwd_delta_kernel(const __nv_bfloat16* __restrict__ out, const __nv_bfloat16* __restrict__ d_out, const float* __restrict__ part,
+                 int nparts, float* __restrict__ delta, float4* __restrict__ dq_acc, int* __restrict__ dq_bad, long long rows, int N, int H) {
+  // delta[b,h,n] = dO[b,n,h,:] . O[b,n,h,:] + part[0][b,h,n] + ... + part[nparts-1][b,h,n].  A warp takes 4 consecutive (b,n,h)
+  // rows at a time: 8 lanes x 16 bytes per 128-byte row (fully coalesced 512-byte requests), 3 shuffles.  The same pass zeroes
+  // the 64-bit dQ accumulator the backward kernel reduces into (64 values per row) and its row flags, which saves a separate
+  // memset node per block of the ViT.
   const int lane = threadIdx.x & 31;
   const long long t = ((long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 4 + (lane >> 3);
   const bool ok = t < rows;
@@ -606,8 +610,8 @@ bwd_delta_kernel(const __nv_bfloat16* __restrict__ out, const __nv_bfloat16* __r
       acc = fmaf(fa.y, fd.y, acc);
     }
     const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    dq_acc[t * (HD / 4) + (lane & 7)] = z;
-    dq_acc[t * (HD / 4) + 8 + (lane & 7)] = z;
+#pragma unroll
+    for (int m = 0; m < 4; ++m) dq_acc[t * (HD / 2) + m * 8 + (lane & 7)] = z;
   }
   acc += __shfl_xor_sync(0xffffffffu, acc, 1);
   acc += __shfl_xor_sync(0xffffffffu, acc, 2);
@@ -616,13 +620,18 @@ bwd_delta_kernel(const __nv_bfloat16* __restrict__ out, const __nv_bfloat16* __r
     const int h = (int)(t % H);
     const long long bn = t / H;
     const int n = (int)(bn % N), b = (int)(bn / N);
-    delta[((size_t)b * H + h) * N + n] = acc;
+    const size_t idx = ((size_t)b * H + h) * N + n;
+    for (int k = 0; k < nparts; ++k) acc += __ldg(part + (size_t)k * rows + idx);
+    delta[idx] = acc;
+    dq_bad[idx] = 0;
   }
 }
 
 __global__ void __launch_bounds__(256)
-bwd_dq_convert_kernel(const float* __restrict__ dq_acc, __nv_bfloat16* __restrict__ d_qkv, int B, int N, int H, float scale) {
-  // dq_acc [B,H,N,64] fp32 -> d_qkv[b,n,0,h,:] bf16 (scaled); one thread per 8 elements
+bwd_dq_convert_kernel(const long long* __restrict__ dq_acc, const int* __restrict__ dq_bad, __nv_bfloat16* __restrict__ d_qkv, int B, int N,
+                      int H, float scale) {
+  // dq_acc [B,H,N,64] 64-bit fixed point -> d_qkv[b,n,0,h,:] bf16 (scaled), NaN for a row whose sum left the fixed-point range
+  // or met a non-finite value (dq_bad); one thread per 8 elements
   const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= (long long)B * H * N * (HD / 8)) return;
   const int c = (int)(t % (HD / 8));
@@ -630,13 +639,20 @@ bwd_dq_convert_kernel(const float* __restrict__ dq_acc, __nv_bfloat16* __restric
   const int n = (int)(row % N);
   const int h = (int)((row / N) % H);
   const int b = (int)(row / ((long long)N * H));
-  const float4* src = reinterpret_cast<const float4*>(dq_acc + row * HD + c * 8);
-  const float4 x = __ldg(src), y = __ldg(src + 1);
+  const longlong2* src = reinterpret_cast<const longlong2*>(dq_acc + row * HD + c * 8);
+  const float sc = __ldg(dq_bad + row) ? __int_as_float(0x7fc00000) : scale * kDqUnfix;    // kDqUnfix * scale is exact
+  float x[8];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const longlong2 q = __ldg(src + j);
+    x[2 * j] = __ll2float_rn(q.x) * sc;
+    x[2 * j + 1] = __ll2float_rn(q.y) * sc;
+  }
   uint4 v;
-  v.x = tc::pack_bf16(x.x * scale, x.y * scale);
-  v.y = tc::pack_bf16(x.z * scale, x.w * scale);
-  v.z = tc::pack_bf16(y.x * scale, y.y * scale);
-  v.w = tc::pack_bf16(y.z * scale, y.w * scale);
+  v.x = tc::pack_bf16(x[0], x[1]);
+  v.y = tc::pack_bf16(x[2], x[3]);
+  v.z = tc::pack_bf16(x[4], x[5]);
+  v.w = tc::pack_bf16(x[6], x[7]);
   *reinterpret_cast<uint4*>(d_qkv + (((size_t)b * N + n) * 3 + 0) * ((size_t)H * HD) + (size_t)h * HD + c * 8) = v;
 }
 
@@ -644,8 +660,10 @@ bwd_dq_convert_kernel(const float* __restrict__ dq_acc, __nv_bfloat16* __restric
 
 extern "C" size_t acr_attn_bwd_bf16_workspace(int B, int N, int H, int D) {
   if (B <= 0 || N <= 0 || H <= 0 || D <= 0) return 0;
-  const size_t rows = (size_t)B * H * N;
-  return acr::align_up(rows * sizeof(float), 256) + acr::align_up(rows * D * sizeof(float), 256);
+  const size_t rows = (size_t)B * H * N, kt = (N + BN - 1) / BN;
+  // delta | 64-bit dQ accumulator | one delta partial plane per key tile | dQ row flags
+  return acr::align_up(rows * sizeof(float), 256) + acr::align_up(rows * D * sizeof(long long), 256) + acr::align_up(kt * rows * sizeof(float), 256) +
+         acr::align_up(rows * sizeof(int), 256);
 }
 
 extern "C" int acr_attn_bwd_bf16(const void* qkv, const void* out, const float* lse, const void* d_out,
@@ -671,40 +689,43 @@ extern "C" int acr_attn_bwd_bf16(const void* qkv, const void* out, const float* 
   ACR_REQUIRE(acr_device_is_sm100(), ACR_E_NOSM100, "acr_attn_bwd_bf16: needs an sm_100 device");
   cudaStream_t st = (cudaStream_t)stream;
   const size_t rows = (size_t)B * H * N;
+  const int qt = (N + BM - 1) / BM, kt = (N + BN - 1) / BN;
   float* delta = (float*)workspace;
-  float* dq_acc = (float*)((char*)workspace + acr::align_up(rows * sizeof(float), 256));
+  long long* dq_acc = (long long*)((char*)workspace + acr::align_up(rows * sizeof(float), 256));
+  float* delta_part = (float*)((char*)dq_acc + acr::align_up(rows * D * sizeof(long long), 256));
+  int* dq_bad = (int*)((char*)delta_part + acr::align_up((size_t)kt * rows * sizeof(float), 256));
   CUtensorMap tmap_qkv, tmap_do, tmap_dq;
   if (int e = make_tmap(&tmap_qkv, qkv, B, N, 3 * H, D)) return e;
   if (int e = make_tmap(&tmap_do, d_out, B, N, H, D)) return e;
-  {   // fp32 dQ accumulator [B*H, N, 64] as (d, n, bh); box = 32 floats (128 B, SWIZZLE_128B) x 128 rows
+  {   // 64-bit dQ accumulator [B*H, N, 64] as (d, n, bh); box = 16 values (128 B, SWIZZLE_128B) x 128 rows
     EncodeTiledFn fn = get_encode_fn();
     ACR_REQUIRE(fn != nullptr, ACR_E_NOSM100, "cuTensorMapEncodeTiled unavailable");
     cuuint64_t dims[3] = {(cuuint64_t)HD, (cuuint64_t)N, (cuuint64_t)B * H};
-    cuuint64_t strides[2] = {(cuuint64_t)HD * 4, (cuuint64_t)N * HD * 4};
-    cuuint32_t box[3] = {32, (cuuint32_t)BM, 1};
+    cuuint64_t strides[2] = {(cuuint64_t)HD * 8, (cuuint64_t)N * HD * 8};
+    cuuint32_t box[3] = {16, (cuuint32_t)BM, 1};
     cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = fn(&tmap_dq, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, dq_acc, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    CUresult r = fn(&tmap_dq, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, dq_acc, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     ACR_REQUIRE(r == CUDA_SUCCESS, ACR_E_INVAL, "cuTensorMapEncodeTiled(dq) failed (%d)", (int)r);
   }
   const float scale_log2 = scale * kLog2e;
-  const int qt = (N + BM - 1) / BM, kt = (N + BN - 1) / BN;
 
-  bwd_delta_kernel<<<(unsigned)((rows + 31) / 32), 256, 0, st>>>((const __nv_bfloat16*)out, (const __nv_bfloat16*)d_out, delta,
-                                                               reinterpret_cast<float4*>(dq_acc), (long long)rows, N, H);
-  if (int e = acr::check_launch("bwd_delta_kernel")) return e;
-  if (g_mean || g_code) {
+  const bool with_g = g_mean || g_code;
+  if (with_g) {
     const size_t smem = sizeof(MeanSmem) + 1024;
     static bool attr_set[64] = {false};
     if (int e = set_max_smem(attn_mean_kernel<1>, smem, attr_set)) return e;
     dim3 grid(kt, qt, B);
     acr::KernelTimer kt_("attn_delta_kernel", st);
-    attn_mean_kernel<1><<<grid, MEAN_THREADS, smem, st>>>(tmap_qkv, lse, const_cast<float*>(g_mean), g_batch_stride, g_row_stride, gc, delta, N, H, scale_log2);
+    attn_mean_kernel<1><<<grid, MEAN_THREADS, smem, st>>>(tmap_qkv, lse, const_cast<float*>(g_mean), g_batch_stride, g_row_stride, gc, delta_part, N, H, scale_log2);
     if (int e = acr::check_launch("attn_mean_kernel<1>")) return e;
   }
-  if (int e = launch_attn_bwd(tmap_qkv, tmap_do, tmap_dq, lse, delta, g_mean, g_batch_stride, g_row_stride, gc, (__nv_bfloat16*)d_qkv, g_row0, B, N, H, scale, st))
+  bwd_delta_kernel<<<(unsigned)((rows + 31) / 32), 256, 0, st>>>((const __nv_bfloat16*)out, (const __nv_bfloat16*)d_out, delta_part,
+                                                               with_g ? kt : 0, delta, reinterpret_cast<float4*>(dq_acc), dq_bad, (long long)rows, N, H);
+  if (int e = acr::check_launch("bwd_delta_kernel")) return e;
+  if (int e = launch_attn_bwd(tmap_qkv, tmap_do, tmap_dq, lse, delta, g_mean, g_batch_stride, g_row_stride, gc, (__nv_bfloat16*)d_qkv, g_row0, dq_bad, B, N, H, scale, st))
     return e;
   const long long nconv = (long long)rows * (HD / 8);
-  bwd_dq_convert_kernel<<<(unsigned)((nconv + 255) / 256), 256, 0, st>>>(dq_acc, (__nv_bfloat16*)d_qkv, B, N, H, scale);
+  bwd_dq_convert_kernel<<<(unsigned)((nconv + 255) / 256), 256, 0, st>>>(dq_acc, dq_bad, (__nv_bfloat16*)d_qkv, B, N, H, scale);
   return acr::check_launch("bwd_dq_convert_kernel");
 }

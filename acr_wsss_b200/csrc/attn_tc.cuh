@@ -12,6 +12,18 @@ constexpr uint32_t TILE_BYTES = BM * HD * 2;
 constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
 constexpr int MEAN_MAX_H = 32;
+// dQ is summed over the key tiles in 64-bit fixed point (value * 2^40, resolution 2^-40): integer addition is associative, so
+// the order in which the key tiles' TMA reduce-adds land does not change a bit of the result.  Range: the host passes the
+// largest per-tile magnitude that kt partials can sum without leaving int64 (dq_fix_limit: 2^(62 - ceil(log2 kt)) in fixed
+// units, i.e. |partial| < 2^19 for N <= 1024); a partial beyond it, or not finite, is not added but marks its query row, and
+// bwd_dq_convert_kernel writes that row of dQ as NaN (a NaN or overflow propagates, as it would through an fp32 sum).
+constexpr float kDqFix = 1099511627776.0f;            // 2^40
+constexpr float kDqUnfix = 1.0f / 1099511627776.0f;   // 2^-40
+inline float dq_fix_limit(int kt) {
+  int lg = 0;
+  while ((1 << lg) < kt) ++lg;
+  return ldexpf(1.0f, 62 - lg);
+}
 
 constexpr uint32_t IDESC_S = tc::idesc_bf16_f32(128, 128, 0, 0);   // S = Q K^T : A, B K-major
 constexpr uint32_t IDESC_PV = tc::idesc_bf16_f32(128, 64, 0, 1);   // O = P V   : A K-major, B = V MN-major
@@ -52,6 +64,6 @@ int set_max_smem(K kernel, size_t bytes, bool* done /* [64] */) {
 // backward kernel launcher (attn_bwd_tc.cu)
 int launch_attn_bwd(const CUtensorMap& tmap_qkv, const CUtensorMap& tmap_do, const CUtensorMap& tmap_dq, const float* lse, const float* delta,
                     const float* g_mean, long long g_bs, long long g_ld, const GCode& gc, __nv_bfloat16* d_qkv, float* g_row0,
-                    int B, int N, int H, float scale, cudaStream_t st);
+                    int* dq_bad, int B, int N, int H, float scale, cudaStream_t st);
 
 }  // namespace acr_attn

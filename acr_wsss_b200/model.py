@@ -193,6 +193,44 @@ class PatchEmbed(nn.Module):
         self.proj = nn.Conv2d(in_chans, embed_dim, kernel_size=patch_size, stride=patch_size)
 
 
+_BILINEAR = {}
+
+
+def _bilinear_matrix(n_in, n_out, device):
+    """[n_out, n_in] weights of F.interpolate(mode="bilinear", align_corners=False) along one axis: output d reads
+    src = (d + 0.5) * n_in / n_out - 0.5 (clamped at 0) from its two neighbours.  Built with device ops, so a first call inside a
+    CUDA-graph capture is captured too; kept for reuse only outside one (a captured tensor holds nothing until the replay)."""
+    key = (n_in, n_out, str(device))
+    m = _BILINEAR.get(key)
+    if m is None:
+        src = ((torch.arange(n_out, dtype=torch.float32, device=device) + 0.5) * (n_in / n_out) - 0.5).clamp(min=0.0)
+        i0 = src.floor()
+        l1 = src - i0
+        i1 = torch.clamp(i0 + 1, max=n_in - 1)
+        cols = torch.arange(n_in, dtype=torch.float32, device=device)
+        m = (cols == i0[:, None]) * (1.0 - l1)[:, None] + (cols == i1[:, None]) * l1[:, None]
+        if not (m.is_cuda and torch.cuda.is_current_stream_capturing()):
+            _BILINEAR[key] = m
+    return m
+
+
+class _ResizeGrid(torch.autograd.Function):
+    """F.interpolate(grid [1,E,g,g], (gs_h, gs_w), mode="bilinear").  The backward is mh^T . grad . mw with the interpolation
+    matrices instead of the library's atomic scatter, whose summation order (and so the gradient's rounding) changes from run
+    to run."""
+
+    @staticmethod
+    def forward(ctx, grid, gs_h, gs_w):
+        ctx.sizes = (grid.shape[-1], gs_h, gs_w)
+        return F.interpolate(grid, size=(gs_h, gs_w), mode="bilinear")
+
+    @staticmethod
+    def backward(ctx, grad):
+        gs_old, gs_h, gs_w = ctx.sizes
+        mh, mw = (_bilinear_matrix(gs_old, n, grad.device).to(grad.dtype) for n in (gs_h, gs_w))
+        return mh.t() @ grad @ mw, None, None
+
+
 def _trunc_normal_(t, std=.02):
     return nn.init.trunc_normal_(t, std=std, a=-2., b=2.)
 
@@ -236,7 +274,7 @@ class VisionTransformer(nn.Module):
         posemb_tok, posemb_grid = posemb[:, :self.start_index], posemb[0, self.start_index:]
         gs_old = int(math.sqrt(len(posemb_grid)))
         posemb_grid = posemb_grid.reshape(1, gs_old, gs_old, -1).permute(0, 3, 1, 2)
-        posemb_grid = F.interpolate(posemb_grid, size=(gs_h, gs_w), mode="bilinear")
+        posemb_grid = _ResizeGrid.apply(posemb_grid, gs_h, gs_w)
         posemb_grid = posemb_grid.permute(0, 2, 3, 1).reshape(1, gs_h * gs_w, -1)
         return torch.cat([posemb_tok, posemb_grid], dim=1)
 

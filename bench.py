@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            this repo's CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference --steps K --warmup W    the reference algorithm's CPU path (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                    also write what the last timed step returned (see dump_outputs)
 
 A "step" = one pass of train_acr.py:127-174 over one synthetic batch: two views forward (ViT-B/16, 448x448, 20
 classes, B=8 per GPU), BCE + all-pairs consistency loss, backward, gradient all-reduce (N>1), SGD step.
@@ -42,6 +43,29 @@ def peaks():
         d = json.load(open(p))
         return {"hbm_gbs": d["hbm_gbs"], "tflops_burst": d["bf16_tflops"], "tflops_sustained": d["bf16_tflops_sustained"], "src": "measured"}
     return {"hbm_gbs": 6650.0, "tflops_burst": 1590.0, "tflops_sustained": 1400.0, "src": "fallback"}
+
+
+DUMP_SAMPLE = 1 << 22       # sampled elements per array: 2 x 16 MB of float32
+
+
+def dump_outputs(out_dir, loss, model):
+    """What a caller of the timed training step receives after its last step, as float32 .npy files in `out_dir`: the returned
+    loss (loss.npy), and one fixed, seeded sample of the updated parameters (params_sample.npy) and of their gradients `p.grad`
+    (grads_sample.npy), both indexed in the concatenation of the trained parameters in model.named_parameters() order, so the
+    files of two builds compare element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    params = [p for _, p in model.named_parameters() if p.requires_grad]
+    n = sum(p.numel() for p in params)
+    idx = torch.randint(0, n, (min(DUMP_SAMPLE, n),), generator=torch.Generator().manual_seed(0)).sort().values.to(params[0].device)
+
+    def sample(ts):
+        return torch.cat([t.detach().reshape(-1).float() for t in ts])[idx].cpu().numpy()
+
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "params_sample.npy"), sample(params))
+    np.save(os.path.join(out_dir, "grads_sample.npy"), sample([p.grad for p in params]))
 
 
 class ClockSampler:
@@ -293,7 +317,14 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_dev = timed(lambda: trainer.step(img_d, lab_d), args.steps)
+    last_loss = [None]
+
+    def train_step():
+        last_loss[0] = trainer.step(img_d, lab_d)
+
+    ms_dev = timed(train_step, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_loss[0], model)      # before the steps below train the model further
 
     def e2e_step():
         # the public API's pipelined step: consume the batch whose pinned-host -> device copy was started one step earlier and
@@ -471,7 +502,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cam", action="store_true", help="skip the secondary CAM-inference measurement")
     ap.add_argument("--profile-range", action="store_true", help="wrap one extra step in cudaProfilerStart/Stop (for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss, parameters and gradients of the last timed step (sampled) as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what this repo's CUDA path computed; it does not apply to --impl reference")
     # stdout carries exactly ONE JSON line: everything libraries print while the bench runs (e.g. NCCL's version banner goes
     # to stdout) is sent to stderr instead, at file-descriptor level, and the line is written to the real stdout at the end
     sys.stdout.flush()

@@ -573,6 +573,50 @@ def test_attention_bf16_backward_vs_oracle(dev, B, N, H, with_g):
     assert rel_err(t2n(st["grad_row0"]), t2n(dP_r[:, :, 0, :])) < BF16_TOL
 
 
+def _bf16_attention_grad(qkv, d_out, G, H):
+    from acr_wsss_b200 import ops
+    q = qkv.clone().requires_grad_(True)
+    out, mean = ops.attention_core(q, H, 64 ** -0.5, None, {"capture_grad": True}, "bf16")
+    loss = (out.float() * d_out.float()).sum()
+    if G is not None:
+        loss = loss + (mean * G).sum()
+    loss.backward()
+    return q.grad
+
+
+def test_attention_bf16_backward_is_identical_run_to_run(dev):
+    """The key tiles' shares of delta and of dQ are summed in a fixed order / in 64-bit fixed point, so repeated backward passes
+    on the same inputs give the same bits (N = 785: seven key tiles per (head, image), on different CTAs)."""
+    B, N, H, D = 2, 785, 12, 64
+    g = torch.Generator().manual_seed(5)
+    qkv = (torch.randn(B, N, 3 * H * D, generator=g) * 1.5).to(torch.bfloat16).to(dev)
+    d_out = torch.randn(B, N, H * D, generator=g).to(torch.bfloat16).to(dev)
+    G = (torch.randn(B, N, N, generator=g) * 0.05).to(dev)
+    grads = [_bf16_attention_grad(qkv, d_out, G, H) for _ in range(3)]
+    assert all(torch.equal(grads[0], x) for x in grads[1:])
+
+
+def test_attention_bf16_backward_propagates_nan_and_overflow(dev):
+    """dQ's fixed-point sum never turns a NaN, or a value beyond its range, into a finite number: such a query row comes out
+    as NaN, and every finite entry matches the fp32 reference."""
+    orc = _orc()
+    B, N, H, D = 1, 300, 2, 64
+    g = torch.Generator().manual_seed(6)
+    qkv = (torch.randn(B, N, 3 * H * D, generator=g) * 1.5).to(torch.bfloat16)
+    d_out = torch.randn(B, N, H * D, generator=g).to(torch.bfloat16)
+    bad = d_out.clone()
+    bad[0, 7, 0] = float("nan")                                  # query row 7 of head 0
+    dq = _bf16_attention_grad(qkv.to(dev), bad.to(dev), None, H).reshape(B, N, 3, H, D)[:, :, 0]
+    assert torch.isnan(dq[0, 7, 0]).all()
+    big = d_out * 2.0 ** 24                                      # dQ far beyond the fixed-point range (|partial| < 2^19 before scaling)
+    dq = _bf16_attention_grad(qkv.to(dev), big.to(dev), None, H).reshape(B, N, 3, H, D)[:, :, 0].float().cpu()
+    ref = orc.attention_core_backward(qkv.float(), H, D ** -0.5, big.float(), None)[0].reshape(B, N, 3, H, D)[:, :, 0]
+    nan = torch.isnan(dq)
+    assert nan.any()
+    diff = (dq - ref).abs()[~nan]
+    assert torch.isfinite(diff).all() and (diff.numel() == 0 or float(diff.max()) <= 2 * BF16_TOL * float(ref.abs().max()))
+
+
 def test_fused_path_accessors_full_maps(dev):
     """Accessor protocol on the fused bf16 path (vision_transformer.py:186-196, DPT/ACR.py:182-183,206): get_attn() and
     get_attn_gradients() return the full [B,H,N,N] maps (recomputed on demand: the kernels keep row 0 only), consistent with the
@@ -934,16 +978,42 @@ def test_trainer_cuda_graph_matches_eager(dev, S, B):
         finals.append(m.cls_head.weight.detach().float().cpu().clone())
         assert abs(tr.opt.param_groups[0]["lr"] - 0.01 * (1 - 4 / 50) ** 0.9) < 1e-9
     assert losses[0][0] > losses[0][-1]                       # it trains
-    # the two modes differ in rounding only (cached bf16 weights + fp32 bias-gradient sums vs autocast, atomics order);
+    # the two modes differ in rounding only (cached bf16 weights + fp32 bias-gradient sums vs autocast);
     # sign() gradients amplify that along the trajectory (measured at S = 64: 0 / 4e-5 / 1e-2 / 3e-2 / 2e-2 relative over the
-    # five steps, the later ones moving by a factor of two with any change of summation order in the kernels -- the dQ
-    # reduce-adds land in a different order on every run), so the first loss is compared tightly, the loss after one complete
-    # update in either mode at 1e-2, and the rest of the trajectory loosely
+    # five steps, the later ones moving by a factor of two with any change of summation order in the kernels), so the first
+    # loss is compared tightly, the loss after one complete update in either mode at 1e-2, and the rest of the trajectory loosely
     assert abs(losses[0][0] - losses[1][0]) <= 2e-3 * abs(losses[1][0]), losses
     assert abs(losses[0][1] - losses[1][1]) <= 1e-2 * abs(losses[1][1]), losses
     for a, b in zip(*losses):
         assert abs(a - b) <= 1e-1 * abs(b), (losses)
     assert rel_err(t2n(finals[0]), t2n(finals[1])) < 5e-2
+
+
+def test_trainer_steps_are_identical_run_to_run(dev):
+    """Two Trainers from the same weights on the same batch take bit-identical CUDA-graph steps at 448x448 (N = 785): losses,
+    gradients and updated weights.  Rounding differences would grow along the trajectory, so this holds only if no sum on the
+    step's path depends on the order in which CTAs finish."""
+    from acr_wsss_b200 import ACR, Trainer, synth
+    orc = _orc()
+    S, B, C = 448, 2, 20
+    sd = orc.synth_state_dict(orc.vit_shapes(768, 12, C), qkv_gain=2.0)
+    img, label = synth.images(B, S).to(dev), synth.labels(B, C).to(dev)
+    runs = []
+    for _ in range(2):
+        m = ACR(C, "vitb", precision="bf16").to(dev)
+        m.load_state_dict(sd)
+        for n, p in m.named_parameters():
+            if n.startswith(("pretrained.model.norm.", "pretrained.model.head.", "scratch.")) or n.endswith("bkg_token"):
+                p.requires_grad_(False)
+        tr = Trainer(m, lr=0.01, max_step=50, alpha=100.0)
+        losses = torch.stack([tr.step(img, label).clone() for _ in range(5)])       # 2 eager warm-ups, capture, 2 replays
+        trained = [p for p in m.parameters() if p.requires_grad]
+        runs.append((losses, [p.detach().clone() for p in trained], [p.grad.clone() for p in trained]))
+        del tr, m
+    (l0, p0, g0), (l1, p1, g1) = runs
+    assert torch.equal(l0, l1), (l0, l1)
+    assert all(torch.equal(a, b) for a, b in zip(g0, g1))
+    assert all(torch.equal(a, b) for a, b in zip(p0, p1))
 
 
 @pytest.mark.parametrize("M,F", [(1, 2), (37, 768), (12560, 3072), (513, 20)])
