@@ -18,14 +18,17 @@ def timeit(fn, iters=10):
     return tot / iters * 1e3
 
 res = {}
-for (B, C, S, it, dil) in [(1, 21, 448, 10, [1, 2, 4, 8, 12, 24]), (8, 21, 448, 10, [1, 2, 4, 8, 12, 24]), (1, 81, 448, 10, [1, 2, 4, 8, 12, 24])]:
-    x = ((synth.smooth_rgb(B, S, S, seed=4) - 120.0) / 58.0).to(dev)
-    mask = synth.probabilities(B, C, S // 16, S // 16, seed=4).to(dev)
+STD = [1, 2, 4, 8, 12, 24]
+# 500 x 375 (a VOC-sized image) times a width that is not a multiple of 4: its rows end in unused cells up to the 16-byte pitch
+for (B, C, H, W, it, dil) in [(1, 21, 448, 448, 10, STD), (8, 21, 448, 448, 10, STD), (1, 81, 448, 448, 10, STD), (1, 21, 500, 375, 10, STD)]:
+    x = ((synth.smooth_rgb(B, H, W, seed=4) - 120.0) / 58.0).to(dev)
+    mask = synth.probabilities(B, C, H // 16, W // 16, seed=4).to(dev)
     pamr = PAMR(it, dil)
     t = timeit(lambda: pamr(x, mask))
-    D = len(dil); HW = S * S
+    D = len(dil); HW = H * W
     alg = B * (HW * (3 * 4 + 8 * D * 4) + it * HW * (8 * D * 4 + 2 * C * 4))
-    res[f"pamr_B{B}_C{C}_us"] = round(t, 1); res[f"pamr_B{B}_C{C}_GBs"] = round(alg / t / 1e3, 1)
+    key = f"pamr_B{B}_C{C}_{H}x{W}"
+    res[f"{key}_us"] = round(t, 1); res[f"{key}_GBs"] = round(alg / t / 1e3, 1)
 for (N, K, S) in ([] if 'pamr' in sys.argv else [(1, 21, 224), (8, 21, 224), (8, 81, 224)]):
     img = synth.smooth_rgb(N, S, S, seed=0).to(dev); ins = synth.probabilities(N, K, S, S, seed=0).to(dev)
     t = timeit(lambda: ops.bilateral_filter(img, ins, 15.0, 50.0))
