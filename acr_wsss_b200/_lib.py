@@ -53,6 +53,8 @@ SIGNATURES = {
     "acr_affinity_refine_tc_workspace": (c_size_t, [c_int, c_int, c_int, c_int]),
     "acr_affinity_refine_tc": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "acr_patch_cam_tc": (c_int, [c_void_p, c_longlong, c_longlong, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "acr_cam_finish": (c_int, [POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int), c_int, c_int, c_int, c_int, c_void_p,
+                               POINTER(c_longlong), c_int, c_void_p, c_longlong, c_void_p, c_size_t, c_void_p]),
     "acr_crf_head_fwd": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "acr_crf_head_bwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "acr_bilinear_up_bwd": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),

@@ -3,8 +3,12 @@
 `infer_cam_image` reproduces the per-image loop body (scales x flips x present classes) with the hot pieces
 on this repo's kernels: head-mean stack (fused attention), GETAM from row-0 quantities, A = sum_l attn[:,l,1:,1:]
 and ONE [Np x Np]x[Np x C'] contraction for all present classes instead of C' matrix-vector products.
-Bilinear resizes are library calls (F.interpolate), exactly the ones the reference makes.
+Bilinear resizes are library calls (F.interpolate), exactly the ones the reference makes.  `infer_cam_batch` runs M images
+per trunk pass and finishes all of them (resizes to each image's own size, flips, sums, normalisation) in one kernel.
 """
+import numbers
+import weakref
+
 import numpy as np
 import torch
 import torch.nn.functional as F
@@ -107,13 +111,16 @@ def _lowres_pass_batch(model, both, idx, n, start_layer, getam_func, aff, t, nor
 
 class _LowresGraph:
     """CUDA graph of _lowres_pass for one (model, input shape, number of present classes, options) key: the pass is ~270
-    launches of small kernels at batch 2 and is CPU-launch bound when run eagerly (8.4 ms per image, 2.8 ms of GPU time)."""
+    launches of small kernels at batch 2 and is CPU-launch bound when run eagerly (8.4 ms per image, 2.8 ms of GPU time).
+    It lives in model._cam_graphs and holds the model weakly: a strong reference would make model and graphs cyclic garbage,
+    and the cyclic collector could then destroy the graphs and free their memory pool in the middle of an unrelated CUDA graph
+    capture, which invalidates that capture.  Without the cycle they go when the last reference to the model does."""
 
     def __init__(self, model, shape, n_present, args, batch=False):
         dev = next(model.parameters()).device
         self.both = torch.empty(shape, device=dev)
         self.idx = torch.zeros(shape[0] * n_present if batch else n_present, device=dev, dtype=torch.long)
-        self.model, self.n, self.args = model, n_present, args
+        self.model, self.n, self.args = weakref.ref(model), n_present, args
         self.fn = _lowres_pass_batch if batch else _lowres_pass
         self.graph = None
         self.calls = 0
@@ -127,14 +134,14 @@ class _LowresGraph:
         if self.graph is None and self.calls <= 2:          # warm up eagerly on the capture stream (lazy inits, cuBLAS workspaces)
             self.stream.wait_stream(cur)
             with torch.cuda.stream(self.stream):
-                out = self.fn(self.model, self.both, self.idx, self.n, *self.args)
+                out = self.fn(self.model(), self.both, self.idx, self.n, *self.args)
             cur.wait_stream(self.stream)
             return out
         if self.graph is None:
             torch.cuda.synchronize()
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph, stream=self.stream):
-                self.out = self.fn(self.model, self.both, self.idx, self.n, *self.args)
+                self.out = self.fn(self.model(), self.both, self.idx, self.n, *self.args)
         self.graph.replay()
         return self.out
 
@@ -249,28 +256,46 @@ def _to_host(t):
     return host.numpy()
 
 
+def _finish_planes(present, sizes):
+    """Plane table of ops.cam_finish for a batch: per image its GETAM planes (copy k = k-th present class), then its patch-CAM
+    planes, packed back to back.  Returns (rows {offset, image, channel, kind, rows, cols}, total elements)."""
+    planes, total = [], 0
+    for m, (rows, cols) in enumerate(sizes):
+        for kind in (0, 1):
+            for k, ci in enumerate(present[m]):
+                planes.append((total, m, ci if kind else k, kind, rows, cols))
+                total += rows * cols
+    return planes, total
+
+
 def infer_cam_batch(model, imgs, labels, out_size, scales=(1,), start_layer=9, getam_func="cam_grad_s", aff=True, t=1,
                     normalize=False, cuda_graph=False):
-    """infer_cam_image for M images of one shape in ONE pass per scale (the reference loops over images, infer_cam.py:122-215):
-    both flips of all images go through the trunk as a batch of 2M, the blocks >= start_layer run on n copies per image
-    (n = the largest number of present classes in the batch; images with fewer classes carry dummy copies that are dropped),
-    one backward, one batched GETAM, one batched affinity contraction.  imgs [M,3,h,w], labels [M,C], out_size (rows, cols)
-    common to the batch.  Returns a list of (cam_dict, patch_cam_dict) per image, same contents as infer_cam_image."""
+    """infer_cam_image for M images of one input shape in ONE pass per scale (the reference loops over images,
+    infer_cam.py:122-215): both flips of all images go through the trunk as a batch of 2M, the blocks >= start_layer run on n
+    copies per image (n = the largest number of present classes in the batch; images with fewer classes carry dummy copies),
+    one backward, one batched GETAM, one batched affinity contraction.  Then ONE kernel (ops.cam_finish) resizes every
+    present class's GETAM map and patch CAM to its image's original size, adds the flips and scales and min-max normalises
+    them; dummy copies are never computed.
+    imgs [M,3,h,w] (the reference resizes every image to crop_size x crop_size first), labels [M,C]; out_size is the
+    original size (rows, cols) of every image, or a sequence of M such pairs when the originals differ.
+    Returns a list of (cam_dict, patch_cam_dict) per image, the same contents as infer_cam_image; the arrays are views of
+    one pinned host buffer.  An image without a present class gets two empty dicts."""
     M, C = labels.shape
     assert imgs.shape[0] == M
-    rows, cols = out_size
+    if len(out_size) == 2 and all(isinstance(v, numbers.Integral) for v in out_size):
+        sizes = [(int(out_size[0]), int(out_size[1]))] * M
+    else:
+        sizes = [(int(r), int(c)) for r, c in out_size]
+        assert len(sizes) == M, "out_size: (rows, cols) or one such pair per image"
     nblocks = len(model.pretrained.model.blocks)
     assert 0 < start_layer < nblocks, "the batched path stops the backward at block start_layer"
     lab_host = labels.tolist()                                   # one device->host read
     present = [[ci for ci in range(C) if lab_host[m][ci] > 1e-5] for m in range(M)]
     n = max(1, max(len(p) for p in present))
-    padded = [p + [p[0] if p else 0] * (n - len(p)) for p in present]            # dummy copies repeat a class; dropped below
-    idx_m = torch.tensor(padded, device=imgs.device, dtype=torch.long)           # [M,n]
-    idx = idx_m.repeat(2, 1).reshape(-1)                                          # sample (v, m), copy k -> class padded[m][k]
+    padded = [p + [p[0] if p else 0] * (n - len(p)) for p in present]            # dummy copies repeat a class; never finished
+    idx = torch.tensor(padded, device=imgs.device, dtype=torch.long).repeat(2, 1).reshape(-1)   # sample (v, m), copy k
     b, c, h, w = imgs.shape
-    sum_cam = torch.zeros(M, n, rows, cols, device=imgs.device)
-    sum_patch = torch.zeros(M, n, rows, cols, device=imgs.device)
-    lab_sel = labels.gather(1, idx_m).view(M, n, 1, 1)
+    cams_s, patch_s, grids, live = [], [], [], {}
     for scale in scales:
         inp = F.interpolate(imgs, size=(int(h * scale), int(w * scale)), mode="bilinear", align_corners=False)
         ph, pw = int((h * scale) // 16), int((w * scale) // 16)
@@ -283,21 +308,21 @@ def infer_cam_batch(model, imgs, labels, out_size, scales=(1,), start_layer=9, g
                 if len(cache) >= 8:
                     cache.clear()
                 cache[key] = _LowresGraph(model, tuple(both.shape), n, args, batch=True)
+            if key in live:            # a replay overwrites the graph's outputs: keep those of the earlier scale
+                j = live[key]
+                patch_s[j], cams_s[j] = patch_s[j].clone(), cams_s[j].clone()
+            live[key] = len(cams_s)
             patch_cam, cams = cache[key].run(both, idx)
         else:
             patch_cam, cams = _lowres_pass_batch(model, both, idx, n, *args)
-        # patch CAM of the (padded) present classes, infer_cam.py:153-158: [2M,Np,C] -> [2,M,n,rows,cols]
-        pc = patch_cam.permute(0, 2, 1).reshape(2, M, C, ph, pw).gather(2, idx_m.view(1, M, n, 1, 1).expand(2, M, n, ph, pw))
-        pc = F.interpolate(pc.reshape(2 * M, n, ph, pw), [rows, cols], mode="bilinear", align_corners=False).view(2, M, n, rows, cols)
-        pc = pc * lab_sel
-        sum_patch += pc[0].flip(-1) + pc[1]
-        # GETAM maps, infer_cam.py:185-187
-        cm = cams.transpose(1, 2).reshape(2 * M * n, 1, ph, pw)
-        cm = F.interpolate(cm, (rows, cols), mode="bilinear", align_corners=True).view(2, M, n, rows, cols)
-        sum_cam += cm[0].flip(-1) + cm[1]
-    norm = torch.stack([normalize_cam(sum_cam[m], 1e-6) for m in range(M)])      # per-class min-max over the image, :202-209
-    pnorm = torch.stack([normalize_cam(sum_patch[m], 1e-5) for m in range(M)])
-    both_out = torch.stack([norm, pnorm])                                         # [2,M,n,rows,cols]
-    host_np = _to_host(both_out)
-    return [({ci: host_np[0, m, k] for k, ci in enumerate(present[m])}, {ci: host_np[1, m, k] for k, ci in enumerate(present[m])})
-            for m in range(M)]
+        patch_s.append(patch_cam)
+        cams_s.append(cams)
+        grids.append((ph, pw))
+    planes, total = _finish_planes(present, sizes)
+    host = _to_host(ops.cam_finish(cams_s, patch_s, grids, labels, planes, total))
+    maps = iter(host[o:o + r * cl].reshape(r, cl) for o, _, _, _, r, cl in planes)
+    out = []
+    for m in range(M):
+        cam_dict = {ci: next(maps) for ci in present[m]}
+        out.append((cam_dict, {ci: next(maps) for ci in present[m]}))
+    return out

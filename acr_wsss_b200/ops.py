@@ -6,6 +6,7 @@ CPU tensors raise.
 """
 import ctypes
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -719,6 +720,28 @@ def affinity_refine_tc(attn, cam, t=1, normalize=False):
     nbytes = _lib.lib().acr_affinity_refine_tc_workspace(B, N, C, int(t))
     ws = torch.empty(nbytes, device=attn.device, dtype=torch.uint8) if nbytes else None
     _call("acr_affinity_refine_tc", int(t), _p(attn), B, L, N, _p(cam), C, int(t), int(bool(normalize)), _p(out), _p(ws), nbytes, _stream())
+    return out
+
+
+def cam_finish(cams, patches, grids, labels, planes, total):
+    """Finish of batched CAM inference for every plane of a batch in one launch (csrc/cam_finish.cu, infer_cam.py:153-215).
+    cams / patches: per scale [2M, ph*pw, n] GETAM maps and [2M, ph*pw, C] patch CAMs (batch index v*M+m, view 0 = flipped
+    input); grids: per scale (ph, pw); labels [M, C]; planes: rows {offset, image, channel, kind (0 GETAM, 1 patch CAM),
+    rows, cols}, see acr_cam_finish in include/acr_b200.h.  Returns the packed fp32 buffer of `total` elements."""
+    _need_cuda(labels, *cams, *patches)
+    ns = len(grids)
+    assert len(cams) == ns and len(patches) == ns
+    cams = [c.contiguous().float() for c in cams]
+    patches = [c.contiguous().float() for c in patches]
+    labels = labels.contiguous().float()
+    M, C = labels.shape
+    table = np.ascontiguousarray(np.asarray(planes, dtype=np.int64).reshape(-1, 6))
+    out = torch.empty(total, device=labels.device, dtype=torch.float32)
+    ws = torch.empty(table.nbytes, device=labels.device, dtype=torch.uint8)
+    _call("acr_cam_finish", 1 if len(table) else 0,
+          (ctypes.c_void_p * ns)(*[c.data_ptr() for c in cams]), (ctypes.c_void_p * ns)(*[c.data_ptr() for c in patches]),
+          (ctypes.c_int * (2 * ns))(*[int(v) for g in grids for v in g]), ns, M, cams[0].shape[-1], C, _p(labels),
+          table.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)), len(table), _p(out), int(total), _p(ws), table.nbytes, _stream())
     return out
 
 

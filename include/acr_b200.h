@@ -35,9 +35,10 @@ const char* acr_last_error_string(void);
 /* 1 when the current device is compute capability 10.x (tcgen05/TMEM/TMA kernels usable). */
 int acr_device_is_sm100(void);
 
-/* Per-kernel device timing (bench.py's roofline): while enabled, the tensor-core attention kernels are bracketed by CUDA
- * event pairs on the launching stream.  acr_profile_read sums the elapsed time of every recorded launch of `kernel`
- * ("attn_fwd_kernel", "attn_mean_kernel", "attn_delta_kernel", "attn_bwd_kernel") after synchronising its events;
+/* Per-kernel device timing (bench.py's roofline): while enabled, the tensor-core attention kernels and the CAM finish kernel
+ * are bracketed by CUDA event pairs on the launching stream.  acr_profile_read sums the elapsed time of every recorded launch
+ * of `kernel` ("attn_fwd_kernel", "attn_mean_kernel", "attn_delta_kernel", "attn_bwd_kernel", "cam_finish_kernel") after
+ * synchronising its events;
  * acr_profile_enable(0) drops the records.  Must be off during CUDA-graph capture. */
 void acr_profile_enable(int on);
 int acr_profile_read(const char* kernel, double* total_ms, long long* launches);
@@ -204,6 +205,29 @@ int acr_affinity_refine_tc(const float* attn, int B, int L, int N, const float* 
  * weight [C,E] and bias [C] (nullable) as nn.Linear stores them; C <= 128.  Same bf16 hi/lo split as above. */
 int acr_patch_cam_tc(const float* tokens, long long tok_batch_stride, long long tok_row_stride, int B, int M, int E,
                      const float* weight, const float* bias, int C, int relu, float* out, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Finish of batched CAM inference, one launch for a whole batch.  Replaces infer_cam.py:153-215 after the low-res maps
+ * (the resizes to the original image size at :156-162 and :185-187, the flips, the sums over scales and views, and the
+ * per-class min-max normalisation of :202,209) for M images whose original sizes may differ.
+ *   scale s (num_scales in 1..8), HOST arrays: cams_host[s] -> cams_s [2M, ph_s*pw_s, n] (GETAM maps, channel-last),
+ *   patch_host[s] -> patch_s [2M, ph_s*pw_s, C] (patch CAMs), grid_host[2s], grid_host[2s+1] = ph_s, pw_s.  Batch index
+ *   v*M + m is view v of image m; view 0 is the horizontally flipped input.
+ *   labels [M,C] (device): label values; a patch-CAM plane of class c of image m is multiplied by labels[m*C + c].
+ *   planes_host: HOST table of num_planes planes (0..65535), 6 long long each {offset, image, channel, kind, rows, cols}:
+ *     kind 0: GETAM plane of copy `channel` (< n) of cams_s, bilinear with align_corners=True, eps 1e-6;
+ *     kind 1: patch-CAM plane of class `channel` (< C) of patch_s, align_corners=False, times the label, eps 1e-5.
+ *   Each plane is written as rows x cols fp32 at out + offset (offset + rows*cols <= out_elems):
+ *   norm(sum over scales, then views with view 0 first, of the bilinear resize to rows x cols, view 0 read at column
+ *   cols-1-c), norm(x) = (x - min) / (max - min + eps) over the plane.  The resize is ATen's upsample_bilinear2d
+ *   arithmetic for an explicit output size.  Deterministic: no atomics.
+ *   Low-res maps of all scales: 2 * sum_s ph_s*pw_s floats <= 200 KB.
+ *   workspace: >= 48 * num_planes bytes, 8-byte aligned; receives a copy of the table on `stream`.
+ * num_planes = 0 launches nothing (planes_host, out and workspace may then be NULL).
+ * ------------------------------------------------------------------------------------------ */
+int acr_cam_finish(const float* const* cams_host, const float* const* patch_host, const int* grid_host, int num_scales,
+                   int M, int n, int C, const float* labels, const long long* planes_host, int num_planes,
+                   float* out, long long out_elems, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Head of the dense-CRF regulariser (BASELINE configs[3]; call shape myTool.py:825-857, loop train_acr_coco.py:137-165):
