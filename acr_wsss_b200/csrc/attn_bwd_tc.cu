@@ -149,7 +149,7 @@ __device__ __forceinline__ void bwd_softmax_tile(BwdSmem& s, uint32_t tS, uint32
       uint64_t dp = f2_pack(__uint_as_float(rd[2 * e]), __uint_as_float(rd[2 * e + 1]));
       if (GMODE == 3) {
         float g0 = ACR_CODE_F(cw[e >> 1], (2 * e) & 3), g1 = ACR_CODE_F(cw[e >> 1], (2 * e + 1) & 3);
-        if (TAIL) {        // bytes past N are row padding (never written by the loss kernel)
+        if (TAIL) {        // bytes past N are row padding: whatever they hold is no gradient
           if (i0 >= nlive) g0 = 0.f;
           if (i0 + 1 >= nlive) g1 = 0.f;
         }

@@ -65,7 +65,7 @@ int acr_attn_fwd_bf16(const void* qkv_bf16, int B, int N, int H, int D, float sc
 /* Backward of the above with the dense affinity-gradient term (SURVEY section 9):
  *   dP_h = dO_h V_h^T + g_mean / H ;  dS_h = P_h * (dP_h - rowsum(P_h * dP_h)) ; dQ,dK,dV as usual.
  * g_mean (nullable) = dLoss/dA-bar for this block: element (b,i,j) at g_mean + b*g_batch_stride + i*g_row_stride + j
- * (a row stride that is a multiple of 4 with a 16-byte aligned base enables 128-bit loads).
+ * (row and batch strides that are multiples of 4 with a 16-byte aligned base enable 128-bit loads on full key tiles).
  * Alternatively (g_mean NULL) the gradient may be given as sign codes from acr_consistency_fwd_bwd: g_code with strides in
  * BYTES (row stride a multiple of 128 and >= the 128-padded N, base 16-byte aligned), the two weights, and an optional
  * DEVICE scalar g_scale multiplying them (NULL = 1; lets autograd's upstream gradient through without a host sync).
@@ -154,7 +154,8 @@ int acr_gelu_bwd_bf16(const void* x_bf16, const void* dy_bf16, void* dx_bf16, in
  * code1/code2 (nullable together; exclusive with g1/g2): the same gradients as one SIGN CODE byte per element, rows of
  * code_row_stride bytes: 0x00 = 0, 0x3F = +w, 0xBF = -w with w = alpha_cls/(B*L*(N-1)) on row 0 and
  * alpha_aff/(B*L*(N-1)^2) elsewhere (the code is the top byte of +-0.5f).  4x less HBM traffic than fp32 gradients;
- * acr_attn_bwd_bf16 consumes them directly.  Padding bytes of a row are not written.
+ * acr_attn_bwd_bf16 consumes them directly.  The padding bytes [N, code_row_stride) of a row are written as 0x00; the
+ * attention backward never reads them as gradient, so any row padding works there.
  * workspace: scratch of acr_consistency_workspace() bytes.
  * ------------------------------------------------------------------------------------------ */
 size_t acr_consistency_workspace(int B, int L, int N);
