@@ -5,6 +5,7 @@ Public surface (mirrors the reference's names for this path):
     acr_consistency_loss, acr_total_loss       (losses.py   <- train_acr.py:140-168)
     affinity_refine, infer_cam_image/_batch    (cam.py      <- infer_cam.py:145-215)
     save_cam_dict, pseudo_label, label_iou     (cam.py      <- infer_cam.py:227-228, evaluation.py:28-67)
+    crf_inference, crf_with_alpha(_batch)      (cam.py      <- tool/imutils.py crf_inference, myTool.py _crf_with_alpha)
     PAMR                                       (pamr.py     <- pamr.py)
     bilateralfilter_batch                      (bilateralfilter.py <- wrapper/bilateralfilter)
     GpuAugment, Prefetcher, augment_params     (data.py     <- myTool.py:1158-1199 get_data_from_chunk_v2)
@@ -14,6 +15,7 @@ from . import _lib, ops  # noqa: F401
 from .model import ACR, Attention, Block, VisionTransformer  # noqa: F401
 from .losses import acr_consistency_loss, acr_total_loss, dense_crf_loss, dense_crf_loss_from_patch_logits  # noqa: F401
 from .cam import affinity_refine, infer_cam_image, infer_cam_batch, normalize_cam, pseudo_label, save_cam_dict, load_cam_dict, label_iou  # noqa: F401
+from .cam import crf_inference, crf_with_alpha, crf_with_alpha_batch  # noqa: F401
 from .pamr import PAMR  # noqa: F401
 from .train import Trainer, PolyOptimizer  # noqa: F401
 from .parallel import GradBuckets, shard_indices  # noqa: F401

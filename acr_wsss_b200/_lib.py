@@ -64,6 +64,9 @@ SIGNATURES = {
     "acr_bilateral_workspace": (c_size_t, [c_int, c_int, c_int, c_int]),
     "acr_bilateral_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_float,
                                     c_void_p, c_size_t, POINTER(c_int), c_void_p]),
+    "acr_dense_crf_workspace": (c_size_t, [c_int, c_int, c_int, c_int]),
+    "acr_dense_crf": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_float, c_float, c_float,
+                              c_float, c_float, c_void_p, c_size_t, c_void_p]),
     "bilateralfilter_batch_b200": (None, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int,
                                           c_int, c_int, c_int, c_int, c_float, c_float]),
 }

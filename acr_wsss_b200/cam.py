@@ -54,6 +54,52 @@ def save_cam_dict(path, cam_dict):
     np.save(path, {int(k): np.ascontiguousarray(v, dtype=np.float32) for k, v in cam_dict.items()})
 
 
+def crf_inference(img, probs, t=10, scale_factor=1, labels=21):
+    """Drop-in for the reference's crf_inference (tool/imutils.py, pydensecrf): img HWC uint8 [H,W,3], probs [labels,H,W]
+    scores -> numpy float32 [labels,H,W], the marginals after t mean-field iterations of a Gaussian (sxy 3/scale_factor,
+    compat 3) and a bilateral kernel (sxy 80/scale_factor, srgb 13, compat 10), on the current CUDA device."""
+    h, w = img.shape[:2]
+    dev = torch.device("cuda", torch.cuda.current_device())
+    image = torch.from_numpy(np.ascontiguousarray(np.asarray(img).transpose(2, 0, 1), dtype=np.float32)).to(dev)[None]
+    scores = torch.from_numpy(np.ascontiguousarray(probs, dtype=np.float32).reshape(labels, h, w)).to(dev)[None]
+    q = ops.dense_crf(image, scores, n_iter=t, sxy_g=3 / scale_factor, compat_g=3, sxy_b=80 / scale_factor, srgb=13, compat_b=10)
+    return q[0].cpu().numpy()
+
+
+def _bg_scores(cam_dict, alpha):
+    """_crf_with_alpha's scores (myTool.py): [(1 - max_c cam)^alpha, cams in dict order]."""
+    v = np.array(list(cam_dict.values()))
+    bg = np.power(1 - np.max(v, axis=0, keepdims=True), alpha)
+    return np.concatenate((bg, v), axis=0)
+
+
+def crf_with_alpha(img, cam_dict, alpha, t=10):
+    """The reference's _crf_with_alpha (myTool.py) for one image: img HWC uint8, cam_dict {class: [H,W]} ->
+    {0: background marginal, class + 1: marginal of class} (numpy float32 [H,W])."""
+    return crf_with_alpha_batch([img], [cam_dict], alpha, t)[0]
+
+
+def crf_with_alpha_batch(imgs, cam_dicts, alpha, t=10):
+    """crf_with_alpha for a list of images of any sizes: images with the same size and the same number of classes go
+    through one ops.dense_crf call; the results are bitwise those of one call per image.  Returns one dict per image."""
+    scores = [_bg_scores(d, alpha) for d in cam_dicts]
+    groups = {}
+    for m, (img, sc) in enumerate(zip(imgs, scores)):
+        groups.setdefault((img.shape[0], img.shape[1], sc.shape[0]), []).append(m)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    out = [None] * len(imgs)
+    for (h, w, c), idx in groups.items():
+        image = torch.from_numpy(np.stack([np.asarray(imgs[m]).transpose(2, 0, 1) for m in idx]).astype(np.float32)).to(dev)
+        probs = torch.from_numpy(np.stack([scores[m] for m in idx]).astype(np.float32)).to(dev)
+        q = ops.dense_crf(image, probs, n_iter=t).cpu().numpy()
+        for j, m in enumerate(idx):
+            res = {0: q[j, 0]}
+            for i, key in enumerate(cam_dicts[m].keys()):
+                res[key + 1] = q[j, i + 1]
+            out[m] = res
+    return out
+
+
 def load_cam_dict(path):
     """evaluation.py:28-29."""
     return np.load(path, allow_pickle=True).item()

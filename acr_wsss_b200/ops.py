@@ -848,3 +848,22 @@ def bilateral_filter(images, ins, sigmargb, sigmaxy, return_lattice_size=False):
     if return_lattice_size:
         return outs, list(msz)
     return outs
+
+
+def dense_crf(images, probs, n_iter=10, sxy_g=3.0, compat_g=3.0, sxy_b=80.0, srgb=13.0, compat_b=10.0, clip=1e-5):
+    """Dense-CRF mean-field inference (densecrf 2.x, Potts over a Gaussian and a bilateral kernel; acr_dense_crf):
+    images [N,3,H,W] (0..255), probs [N,C,H,W] scores (unary -log(max(P, clip)); they need not sum to 1) -> Q [N,C,H,W],
+    the marginals after n_iter iterations.  Deterministic; capturable in a CUDA graph (the workspace is allocated here)."""
+    _need_cuda(images, probs)
+    N, C, H, W = probs.shape
+    assert images.shape == (N, 3, H, W)
+    images = images.contiguous().float()
+    probs = probs.contiguous().float()
+    q = torch.empty_like(probs)
+    wsb = _lib.lib().acr_dense_crf_workspace(N, C, H, W)
+    ws = torch.empty(wsb + 256, device=probs.device, dtype=torch.uint8)
+    off = (-ws.data_ptr()) % 256
+    _call("acr_dense_crf", (11 + 8 * int(n_iter)) * ((N + 7) // 8), _p(images), _p(probs), _p(q), N, C, H, W, int(n_iter),
+          float(sxy_g), float(compat_g), float(sxy_b), float(srgb), float(compat_b), float(clip),
+          ctypes.c_void_p(ws.data_ptr() + off), wsb, _stream())
+    return q

@@ -275,6 +275,23 @@ void bilateralfilter_batch_b200(const float* images_host, int len_images, const 
                                 float* outs_host, int len_outs,
                                 int N, int K, int H, int W, float sigmargb, float sigmaxy);
 
+/* ------------------------------------------------------------------------------------------
+ * Dense-CRF mean-field inference: densecrf 2.x as tool/imutils.py crf_inference drives it (a Potts model over a Gaussian
+ * kernel on (x/sxy_g, y/sxy_g) and a bilateral kernel on (x/sxy_b, y/sxy_b, r/srgb, g/srgb, b/srgb), both permutohedral,
+ * DIAG_KERNEL + NORMALIZE_SYMMETRIC).  DEVICE buffers: images [N,3,H,W] in 0..255, probs [N,C,H,W] scores (need not sum
+ * to 1; unary = -log(max(P, clip))), q_out [N,C,H,W] the marginals after n_iter iterations (n_iter = 0: softmax of the
+ * clipped log-scores).  PSA defaults: sxy_g = 3, compat_g = 3, sxy_b = 80, srgb = 13, compat_b = 10, clip = 1e-5.
+ * 1 <= C <= 96, 6*H*W < 2^28, sigmas finite and > 0 (small enough sigmas for the image size are rejected: lattice keys are
+ * int16), compat finite, clip in (0, 1].  workspace: acr_dense_crf_workspace() bytes, 256-byte aligned.
+ * Deterministic (two calls, or an image alone and inside a batch, give the same bits); no host synchronisation and no
+ * allocation, so the call can be captured in a CUDA graph.  A splat value outside the fixed-point range makes that image's
+ * q_out NaN.
+ * ------------------------------------------------------------------------------------------ */
+size_t acr_dense_crf_workspace(int N, int C, int H, int W);
+int acr_dense_crf(const float* images, const float* probs, float* q_out, int N, int C, int H, int W, int n_iter,
+                  float sxy_g, float compat_g, float sxy_b, float srgb, float compat_b, float clip,
+                  void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
