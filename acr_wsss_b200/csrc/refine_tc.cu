@@ -268,7 +268,8 @@ extern "C" int acr_affinity_refine_tc(const float* attn, int B, int L, int N, co
                                       float* out, void* workspace, size_t workspace_bytes, void* stream) {
   ACR_REQUIRE(attn && cam && out, ACR_E_INVAL, "acr_affinity_refine_tc: null pointer");
   ACR_REQUIRE(B > 0 && B <= 65535 && L > 0 && N > 1 && C > 0 && t >= 1, ACR_E_INVAL, "acr_affinity_refine_tc: bad shape");
-  ACR_REQUIRE(C + (normalize ? 1 : 0) <= NC_MAX, ACR_E_INVAL, "acr_affinity_refine_tc: at most %d classes per call", NC_MAX - 1);
+  ACR_REQUIRE(C + (normalize ? 1 : 0) <= NC_MAX, ACR_E_INVAL, "acr_affinity_refine_tc: C + normalize must be <= %d (C = %d, normalize = %d)",
+              NC_MAX, C, normalize ? 1 : 0);
   ACR_REQUIRE(t == 1 || (workspace && ((uintptr_t)workspace & 255) == 0 && workspace_bytes >= acr_affinity_refine_tc_workspace(B, N, C, t)),
               ACR_E_NOMEM, "acr_affinity_refine_tc: t > 1 needs acr_affinity_refine_tc_workspace() bytes, 256-byte aligned");
   ACR_REQUIRE(acr_device_is_sm100(), ACR_E_NOSM100, "acr_affinity_refine_tc: needs an sm_100 device");
