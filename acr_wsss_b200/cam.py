@@ -186,7 +186,7 @@ class _LowresGraph:
         if self.graph is None:
             torch.cuda.synchronize()
             self.graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(self.graph, stream=self.stream):
+            with ops.cuda_graph_capture(self.graph, self.stream):
                 self.out = self.fn(self.model(), self.both, self.idx, self.n, *self.args)
         self.graph.replay()
         return self.out

@@ -155,6 +155,8 @@ extern "C" int acr_attn_fwd_f32(const float* qkv, int B, int N, int H, int D, fl
   ACR_REQUIRE(qkv && P && out, ACR_E_INVAL, "acr_attn_fwd_f32: null pointer");
   ACR_REQUIRE(B > 0 && N > 0 && H > 0 && D > 0, ACR_E_INVAL, "acr_attn_fwd_f32: bad shape");
   ACR_REQUIRE((long long)B * H * N < (1ll << 31) && (long long)B * H <= 65535, ACR_E_INVAL, "acr_attn_fwd_f32: batch too large");
+  ACR_REQUIRE(attn_mean == nullptr || (mean_batch_stride >= 0 && (B == 1 || mean_batch_stride >= (long long)N * N)), ACR_E_INVAL,
+              "acr_attn_fwd_f32: mean_batch_stride %lld < N*N: the images' maps would overlap", mean_batch_stride);
   cudaStream_t st = (cudaStream_t)stream;
   const long long E = (long long)H * D, E3 = 3 * E, NN = (long long)N * N;
   const Mat lq{N * E3, D, E3, 1};                 // Q(i,d)

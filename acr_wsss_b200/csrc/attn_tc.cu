@@ -549,6 +549,8 @@ extern "C" int acr_attn_fwd_bf16(const void* qkv, int B, int N, int H, int D, fl
   ACR_REQUIRE(B <= 65535 && H <= MEAN_MAX_H, ACR_E_INVAL, "acr_attn_fwd_bf16: B <= 65535 and H <= %d required", MEAN_MAX_H);
   ACR_REQUIRE(((uintptr_t)qkv & 15) == 0 && ((uintptr_t)out & 15) == 0, ACR_E_ALIGN, "acr_attn_fwd_bf16: qkv/out must be 16-byte aligned");
   ACR_REQUIRE(p_row0 == nullptr || attn_mean != nullptr, ACR_E_INVAL, "acr_attn_fwd_bf16: p_row0 needs attn_mean");
+  ACR_REQUIRE(attn_mean == nullptr || (mean_batch_stride >= 0 && (B == 1 || mean_batch_stride >= (long long)N * N)), ACR_E_INVAL,
+              "acr_attn_fwd_bf16: mean_batch_stride %lld < N*N: the images' maps would overlap", mean_batch_stride);
   ACR_REQUIRE(acr_device_is_sm100(), ACR_E_NOSM100, "acr_attn_fwd_bf16: needs an sm_100 device");
   cudaStream_t st = (cudaStream_t)stream;
   CUtensorMap tmap;

@@ -4,7 +4,9 @@ PyTorch is used here for device memory, streams and autograd bookkeeping only; e
 below is one of the hand-written sm_100a kernels in acr_wsss_b200/csrc.  No CPU fallback exists:
 CPU tensors raise.
 """
+import contextlib
 import ctypes
+import gc
 
 import numpy as np
 import torch
@@ -53,6 +55,23 @@ class direct_grads:
     def __exit__(self, *exc):
         global DIRECT_GRADS
         DIRECT_GRADS = self.prev
+
+
+@contextlib.contextmanager
+def cuda_graph_capture(graph, stream):
+    """torch.cuda.graph(graph, stream=stream) with Python's cycle collector kept out of the capture.  A model or Trainer the
+    caller has dropped lives on in reference cycles until the collector runs; a collection inside a capture would destroy its
+    CUDA graphs, streams and graph memory pool there, which invalidates the capture (cudaErrorStreamCaptureInvalidated at
+    capture_end).  So dead cycles are collected before capture_begin and the collector stays off until capture_end."""
+    gc.collect()
+    enabled = gc.isenabled()
+    gc.disable()
+    try:
+        with torch.cuda.graph(graph, stream=stream):
+            yield
+    finally:
+        if enabled:
+            gc.enable()
 
 
 def _call(name, nlaunch, *args):

@@ -298,10 +298,10 @@ class Trainer:
         if self._g_fb is None:
             torch.cuda.synchronize()
             self._g_fb = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(self._g_fb, stream=self._side):
+            with ops.cuda_graph_capture(self._g_fb, self._side):
                 self._loss = self._forward_backward(img, label)
             self._g_opt = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(self._g_opt, stream=self._side):
+            with ops.cuda_graph_capture(self._g_opt, self._side):
                 self.opt.update()
             self._g_fb.replay()              # the capture itself did not execute the step
         else:

@@ -51,7 +51,8 @@ int acr_profile_read(const char* kernel, double* total_ms, long long* launches);
  * (s=0 q, 1 k, 2 v) -- exactly the buffer the reference reshapes at vision_transformer.py:200.
  * out is [B,N,H*D] (the layout proj consumes, vision_transformer.py:211).
  * attn_mean points at slot l of the [B,L,N,N] fp32 stack: image b's N x N map starts at
- * attn_mean + b*mean_batch_stride (elements); rows are dense (stride N).  May be NULL.
+ * attn_mean + b*mean_batch_stride (elements); rows are dense (stride N).  May be NULL.  mean_batch_stride must not be
+ * negative and, for B > 1, at least N*N (the images' maps must not overlap); otherwise the call fails with ACR_E_INVAL.
  * p_row0 (nullable) receives the per-head softmax row of the cls token, [B,H,N] fp32 (GETAM, a8).
  * ------------------------------------------------------------------------------------------ */
 

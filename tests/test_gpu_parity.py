@@ -1140,3 +1140,56 @@ def test_trainer_prefetch_pipeline_matches_plain_steps(dev):
     for a, b in zip(*losses):
         assert abs(a - b) <= 2e-2 * abs(b), losses
     assert abs(losses[0][0] - losses[1][0]) <= 1e-6 * abs(losses[0][0]), losses     # first step: identical inputs and weights
+
+
+def test_trainer_capture_keeps_the_garbage_collector_out(dev):
+    """A Trainer its caller dropped is freed by Python's cycle collector.  A collection inside the next Trainer's CUDA-graph
+    capture would destroy the old graphs and their memory pool there and invalidate the capture, so whether a second Trainer
+    works would depend on when the collector happens to run.  With the collector set to run on almost every allocation, no
+    collection may start while the step is being captured, and the dropped Trainer must be gone once the capture is done."""
+    import gc
+    import math
+    import weakref
+    from acr_wsss_b200 import ACR, Trainer, synth
+    orc = _orc()
+    S, B, C = 64, 2, 20
+    sd = orc.synth_state_dict(orc.vit_shapes(768, 12, C), qkv_gain=2.0)
+    img, lab = synth.images(B, S, seed=0).to(dev), synth.labels(B, C, seed=0).to(dev)
+    during = []
+
+    def watch(phase, info):
+        if phase == "start" and torch.cuda.is_current_stream_capturing():
+            during.append(info["generation"])
+
+    def trainer():
+        m = ACR(C, "vitb", precision="bf16").to(dev)
+        m.load_state_dict(sd)
+        return Trainer(m, lr=0.01, max_step=50, alpha=100.0)
+
+    enabled, threshold = gc.isenabled(), gc.get_threshold()
+    gc.disable()                   # the dropped Trainer stays in its reference cycles until the step below
+    try:
+        old = trainer()
+        for _ in range(3):
+            old.step(img, lab)     # two eager warm-up steps, then the capture
+        gone = weakref.ref(old)
+        del old
+        assert gone() is not None
+        tr = trainer()
+        for _ in range(2):
+            tr.step(img, lab)
+        gc.callbacks.append(watch)
+        gc.set_threshold(1, 1, 1)
+        gc.enable()
+        loss = float(tr.step(img, lab))
+    finally:
+        if watch in gc.callbacks:
+            gc.callbacks.remove(watch)
+        gc.set_threshold(*threshold)
+        if enabled:
+            gc.enable()
+        else:
+            gc.disable()
+    assert not during, "collections of generations %s ran inside the capture" % sorted(set(during))
+    assert gone() is None
+    assert math.isfinite(loss)
