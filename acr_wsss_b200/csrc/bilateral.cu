@@ -243,7 +243,7 @@ lattice_slice_kernel(const float* __restrict__ values_img0, int K, int HW, float
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int q = lane % G, lp = lane / G;
   constexpr int kPixPerWarp = kPixTile / 8;
-  for (int qq = q; qq < Q; qq += G) {                  // (one trip unless K > 128)
+  for (int qq = q; qq < Q; qq += G) {                  // (one trip: G >= Q = Kp/4 <= 24 for every K <= 96)
     for (int it = 0; it < kPixPerWarp / ppw; ++it) {
       const int p = warp * kPixPerWarp + it * ppw + lp;
       const int pix = p0 + p;

@@ -246,7 +246,8 @@ extern "C" int acr_bilinear_up_bwd(const float* d_up, int planes, int P, int S, 
 
 extern "C" int acr_crf_head_fwd(const float* logits, int B, int P, int C, int S, float* seg, void* stream) {
   ACR_REQUIRE(logits && seg, ACR_E_INVAL, "acr_crf_head_fwd: null pointer");
-  ACR_REQUIRE(B > 0 && B <= 65535 && P > 0 && C > 0 && S >= 2 && (S % 2) == 0 && S / 2 <= 65535, ACR_E_INVAL, "acr_crf_head_fwd: bad shape (S even)");
+  ACR_REQUIRE(B > 0 && B <= 65535 && P > 0 && P <= S && C > 0 && S >= 2 && (S % 2) == 0 && S / 2 <= 65535, ACR_E_INVAL,
+              "acr_crf_head_fwd: bad shape (S even, P <= S)");
   const int h = S / 2;
   crf_head_fwd_kernel<<<dim3((h + 127) / 128, h, B), 128, 0, (cudaStream_t)stream>>>(logits, P, C, S, (float)P / (float)S, seg);
   return acr::check_launch("crf_head_fwd_kernel");
@@ -254,7 +255,8 @@ extern "C" int acr_crf_head_fwd(const float* logits, int B, int P, int C, int S,
 
 extern "C" int acr_crf_head_bwd(const float* logits, const float* g_seg, int B, int P, int C, int S, float* d_up, void* stream) {
   ACR_REQUIRE(logits && g_seg && d_up, ACR_E_INVAL, "acr_crf_head_bwd: null pointer");
-  ACR_REQUIRE(B > 0 && B <= 65535 && P > 0 && C > 0 && S >= 2 && (S % 2) == 0 && S <= 65535, ACR_E_INVAL, "acr_crf_head_bwd: bad shape (S even)");
+  ACR_REQUIRE(B > 0 && B <= 65535 && P > 0 && P <= S && C > 0 && S >= 2 && (S % 2) == 0 && S <= 65535, ACR_E_INVAL,
+              "acr_crf_head_bwd: bad shape (S even, P <= S)");
   const int h = S / 2;
   crf_head_bwd_kernel<<<dim3((h + 127) / 128, h, B), 128, 0, (cudaStream_t)stream>>>(logits, g_seg, P, C, S, (float)P / (float)S, d_up);
   return acr::check_launch("crf_head_bwd_kernel");

@@ -237,7 +237,8 @@ int acr_cam_finish(const float* const* cams_host, const float* const* patch_host
  *   logits [B,P*P,C] fp32 channel-last (cls_head(layer_4[:,1:]), DPT/ACR.py:133-134)
  *   seg    [B,C+1,S/2,S/2] = bilinear_down_0.5( softmax_k([0, bilinear_up(logits -> SxS)]) ), both align_corners=False
  * Backward: g_seg [B,C+1,S/2,S/2] -> d_up [B,C,S,S] = gradient with respect to the up-sampled logits (fold it to patch
- * resolution with the bilinear backward).  S even.
+ * resolution with the bilinear backward).  S even, 1 <= P <= S (the model up-samples; P > S is rejected, so the backward
+ * never meets a shape the bilinear backward below does not take).
  * ------------------------------------------------------------------------------------------ */
 int acr_crf_head_fwd(const float* logits, int B, int P, int C, int S, float* seg, void* stream);
 int acr_crf_head_bwd(const float* logits, const float* g_seg, int B, int P, int C, int S, float* d_up, void* stream);

@@ -99,9 +99,11 @@ static void embed(const float* f, const float* scale, int16_t keys[DV][DF], floa
   }
 }
 
-/* One image: image [3,H,W] in 0..255, in/out [K,H,W].  Returns the number of lattice vertices M. */
-int permuto_oracle_image(const float* image, const float* in, float* out, int K, int H, int W,
-                         float sigmargb, float sigmaxy) {
+/* One image: image [3,H,W] in 0..255, in/out [K,H,W].  Returns the number of lattice vertices M (K = 0: the lattice only,
+ * in/out are not read).  skip_blur_axis in 0..DF leaves that one of the d+1 blur passes out -- a deliberately wrong filter
+ * the tests use to show that they notice a missing pass; -1 is the filter. */
+int permuto_oracle_image_variant(const float* image, const float* in, float* out, int K, int H, int W,
+                                 float sigmargb, float sigmaxy, int skip_blur_axis) {
   const int HW = H * W, HWpad = (HW + 3) / 4 * 4;   /* the reference pads the last group of 4 with zero features */
   float scale[DF];
   const float inv_std_dev = (float)(sqrt(2.0 / 3.0) * (DF + 1));
@@ -158,6 +160,7 @@ int permuto_oracle_image(const float* image, const float* in, float* out, int K,
     for (int i = 0; i < HW; i++)
       for (int r = 0; r < DV; r++) val[offs[(size_t)i * DV + r] + 1] += bary[(size_t)i * DV + r] * ip[i];
     for (int j = 0; j < DV; j++) {
+      if (j == skip_blur_axis) continue;
       for (int v = 0; v < M; v++) {
         float a = val[n1[(size_t)j * M + v] + 1], b = val[n2[(size_t)j * M + v] + 1];
         nval[v + 1] = val[v + 1] + 0.5f * (a + b);
@@ -175,6 +178,11 @@ int permuto_oracle_image(const float* image, const float* in, float* out, int K,
   }
   free(val); free(nval); free(n1); free(n2); free(offs); free(bary); free(m.slots); free(m.keys);
   return M;
+}
+
+int permuto_oracle_image(const float* image, const float* in, float* out, int K, int H, int W,
+                         float sigmargb, float sigmaxy) {
+  return permuto_oracle_image_variant(image, in, out, K, H, W, sigmargb, sigmaxy, -1);
 }
 
 /* Same argument order as the SWIG export bilateralfilter_batch (bilateralfilter.hpp:12). */
