@@ -5,6 +5,9 @@
 
 namespace {
 
+// max(v, 0) that keeps a NaN, as torch's clamp(min=0) and relu do (fmaxf would return 0).
+__device__ __forceinline__ float relu_nan(float v) { return v < 0.f ? 0.f : v; }
+
 // One thread per token j, blockIdx.y = sample.  p/g: [L,S,H,N] (S = 1 for the single-image entry).  See acr_b200.h for `func`.
 __global__ void __launch_bounds__(256)
 getam_row0_kernel(const float* __restrict__ p, const float* __restrict__ g, int S, int L, int H, int N,
@@ -21,8 +24,8 @@ getam_row0_kernel(const float* __restrict__ p, const float* __restrict__ g, int 
     for (int h = 0; h < H; ++h) {
       const long long o = (((long long)l * S + s) * H + h) * N + j;
       const float gv = g[o];
-      pos_g += fmaxf(gv, 0.f);
-      if (func >= 2) pos_gp += fmaxf(gv * p[o], 0.f);
+      pos_g += relu_nan(gv);
+      if (func >= 2) pos_gp += relu_nan(gv * p[o]);
     }
     pos_g *= invH;
     pos_gp *= invH;
@@ -36,7 +39,7 @@ getam_row0_kernel(const float* __restrict__ p, const float* __restrict__ g, int 
     if (cam_rows) cam_rows[(long long)l * N + j] = c;
     if (l >= start_layer) total += c;
   }
-  if (j >= skip) cam_out[j - skip] = fmaxf(total, 0.f);
+  if (j >= skip) cam_out[j - skip] = relu_nan(total);
 }
 
 // A[b,i,:] = sum_l attn[b,l,i+1,1:] (optionally divided by its row sum).  One CTA per (b,i).

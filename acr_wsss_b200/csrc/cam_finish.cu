@@ -7,10 +7,11 @@
 //   1. stage the low-res rows its band samples, both views of every scale, in shared memory (a gather of one channel);
 //   2. bilinear samples with ATen's upsample_bilinear2d arithmetic for an explicit output size, summed in the reference's
 //      order (scales in order, flipped view first), written to the output; band min / max on the side;
-//   3. min / max of the plane through distributed shared memory (exact, so independent of order);
+//   3. min / max of the plane through distributed shared memory (exact, so independent of order); the max keeps a NaN,
+//      so a plane with a NaN pixel comes out all NaN, as normalize_cam's amin / amax make it;
 //   4. every thread normalises the values it wrote itself: (x - min) / (max - min + eps).
 // No atomics, no cross-CTA float sums: two calls give bitwise-identical output.
-#include "common.cuh"
+#include "attn_tc.cuh"      // acr_attn::set_max_smem
 #include <cooperative_groups.h>
 
 namespace cg = cooperative_groups;
@@ -57,6 +58,8 @@ __device__ __forceinline__ Tap axis_tap(int in, float scale, int dst, bool align
   t.l0 = 1.f - t.l1;
   return t;
 }
+// max that returns a NaN operand (fmaxf returns the other one)
+__device__ __forceinline__ float max_nan(float a, float b) { return (a > b || a != a) ? a : b; }
 
 __global__ void __cluster_dims__(kCluster, 1, 1) __launch_bounds__(kThreads)
 cam_finish_kernel(const __grid_constant__ Params p) {
@@ -138,11 +141,12 @@ cam_finish_kernel(const __grid_constant__ Params p) {
         }
       plane[(long long)r * cols + c] = acc;
       mn = fminf(mn, acc);
-      mx = fmaxf(mx, acc);
+      mx = max_nan(mx, acc);
     }
   }
   mn = -acr::warp_max(-mn);
-  mx = acr::warp_max(mx);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = max_nan(mx, __shfl_xor_sync(0xffffffffu, mx, o));
   if (lane == 0) {
     s_red[0][warp] = mn;
     s_red[1][warp] = mx;
@@ -151,7 +155,7 @@ cam_finish_kernel(const __grid_constant__ Params p) {
   if (threadIdx.x == 0) {
     for (int w = 1; w < kThreads / 32; ++w) {
       mn = fminf(mn, s_red[0][w]);
-      mx = fmaxf(mx, s_red[1][w]);
+      mx = max_nan(mx, s_red[1][w]);
     }
     s_band = make_float2(mn, mx);
   }
@@ -161,10 +165,10 @@ cam_finish_kernel(const __grid_constant__ Params p) {
   for (int q = 0; q < kCluster; ++q) {
     const float2 b = *cluster.map_shared_rank(&s_band, q);
     mn = fminf(mn, b.x);
-    mx = fmaxf(mx, b.y);
+    mx = max_nan(mx, b.y);
   }
   cluster.sync();                                      // nobody leaves while its (min, max) is still being read
-  const float den = (mx - mn) + (patch ? 1e-5f : 1e-6f);
+  const float den = (mx - mn) + (patch ? 1e-5f : 1e-6f);      // NaN when the plane holds one
   for (int r = r0 + warp; r < r1; r += kThreads / 32)
     for (int c = lane; c < cols; c += 32) {
       float* q = plane + (long long)r * cols + c;      // written by this thread above
@@ -212,15 +216,9 @@ extern "C" int acr_cam_finish(const float* const* cams_host, const float* const*
   p.planes = (const long long*)workspace;
   p.labels = labels;
   p.out = out;
+  // whatever `smem` is: the kernel's static shared memory counts against the same 48 KB default as the dynamic size
   static bool attr_set[64] = {false};
-  if (smem > 48 * 1024) {
-    int dev = 0;
-    ACR_CUDA(cudaGetDevice(&dev));
-    if (!(dev >= 0 && dev < 64 && attr_set[dev])) {
-      ACR_CUDA(cudaFuncSetAttribute(cam_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
-      if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
-  }
+  if (int e = acr_attn::set_max_smem(cam_finish_kernel, kMaxSmem, attr_set)) return e;
   acr::KernelTimer kt_("cam_finish_kernel", st);
   cam_finish_kernel<<<dim3(kCluster, num_planes), kThreads, smem, st>>>(p);
   return acr::check_launch("cam_finish_kernel");

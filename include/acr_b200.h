@@ -171,7 +171,9 @@ int acr_consistency_fwd_bwd(const float* attn1, const float* attn2, int B, int L
  * reaches the result (row 0 of each block's map).  p_row0/g_row0: [L,H,N] fp32 for ONE image
  * (per-block, per-head cls-token row of P and of dP).  func: 0 'grad', 1 'grad_s', 2 'cam_grad',
  * 3 'cam_grad_s'.  skip = 1 (2 for the distilled DeiT variant).  cam_out [N-skip] fp32.
- * cam_rows (nullable) [L,N] receives each block's c_l row 0.
+ * cam_rows (nullable) [L,N] receives each block's c_l row 0.  The clamps keep NaN, as clamp(min=0) / relu do: a NaN in
+ * g_row0, or in g*p for the cam_grad funcs (a NaN in p_row0, inf * 0), makes that token's c_l NaN, and its CAM too if
+ * l >= start_layer.
  * ------------------------------------------------------------------------------------------ */
 int acr_getam_row0(const float* p_row0, const float* g_row0, int L, int H, int N,
                    int start_layer, int func, int skip,
@@ -222,7 +224,8 @@ int acr_patch_cam_tc(const float* tokens, long long tok_batch_stride, long long 
  *   Each plane is written as rows x cols fp32 at out + offset (offset + rows*cols <= out_elems):
  *   norm(sum over scales, then views with view 0 first, of the bilinear resize to rows x cols, view 0 read at column
  *   cols-1-c), norm(x) = (x - min) / (max - min + eps) over the plane.  The resize is ATen's upsample_bilinear2d
- *   arithmetic for an explicit output size.  Deterministic: no atomics.
+ *   arithmetic for an explicit output size.  A plane whose sum holds a NaN is written as all NaN (amin / amax propagate
+ *   it in the reference's normalisation).  Deterministic: no atomics.
  *   Low-res maps of all scales: 2 * sum_s ph_s*pw_s floats <= 200 KB.
  *   workspace: >= 48 * num_planes bytes, 8-byte aligned; receives a copy of the table on `stream`.
  * num_planes = 0 launches nothing (planes_host, out and workspace may then be NULL).

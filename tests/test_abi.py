@@ -76,6 +76,15 @@ def test_invalid_arguments_are_rejected_before_any_launch():
     assert L.acr_colsum_bf16(al, 4, 7, al, 0, al, 1 << 20, None) == -1                    # F odd
     tot, cnt = ctypes.c_double(), ctypes.c_longlong()
     assert L.acr_profile_read(None, ctypes.byref(tot), ctypes.byref(cnt)) == -1
+    # GETAM row 0, one image and a batch of S samples: L = 12, H = 12, N = 785
+    ok = dict(p=al, g=al, start=0, func=0, skip=1, out=al)
+    for over in (dict(p=None), dict(g=None), dict(out=None), dict(start=-1), dict(start=12), dict(func=4), dict(skip=0),
+                 dict(skip=785)):
+        x = dict(ok, **over)
+        assert L.acr_getam_row0(x["p"], x["g"], 12, 12, 785, x["start"], x["func"], x["skip"], x["out"], None, None) == -1, over
+        assert L.acr_getam_row0_batch(x["p"], x["g"], 48, 12, 12, 785, x["start"], x["func"], x["skip"], x["out"], None) == -1, over
+    for S in (0, 65536):
+        assert L.acr_getam_row0_batch(al, al, S, 12, 12, 785, 0, 0, 1, al, None) == -1, S
 
 
 def test_pseudo_label_writer_roundtrip(tmp_path):

@@ -45,6 +45,7 @@ def test_cam_finish_rejects_invalid_arguments_before_any_launch():
         "no scale": dict(ns=0), "9 scales": dict(ns=9),
         "M < 1": dict(M=0), "n < 1": dict(n=0), "C < 1": dict(C=0),
         "grid rows 0": dict(grid=[7, 7, 0, 14]), "grid cols < 0": dict(grid=[7, -1, 14, 14]),
+        "low-res maps of 206080 bytes > 200 KB": dict(grid=[160, 161], ns=1),
         "negative plane count": dict(num_planes=-1),
         "null table": dict(planes=None, num_planes=4), "null out": dict(out=None), "null workspace": dict(ws=None),
         "rows 0": dict(planes=_plane(0, rows=0)), "cols < 0": dict(planes=_plane(2, cols=-7)),
