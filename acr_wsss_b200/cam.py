@@ -122,6 +122,106 @@ def label_iou(pred_labels, gt_labels, num_cls=21):
     return iou, float(np.mean(iou))
 
 
+def _above(h):
+    """[..., t] = sum over j > t of h[..., j], for t = 0..J-2 (int64 on the device: exact)."""
+    return h.flip(-1).cumsum(-1).flip(-1)[..., 1:]
+
+
+def _curve_counts(counts, num_cls, num_thresholds):
+    """ops.cam_label_counts' counters -> label_iou's P, T, TP at every threshold, int64 [T, num_cls] each.  A pixel with
+    best class c and j thresholds below its value is labelled c at thresholds 0..j-1 and background above; so class c >= 1
+    gets the pixels with j > t, and background the rest of the valid pixels."""
+    K, T = num_cls, num_thresholds
+    n = (K - 1) * (T + 1)
+    by_class = counts[:n].view(K - 1, T + 1)
+    hit = counts[n:2 * n].view(K - 1, T + 1)
+    bg_gt = counts[2 * n:2 * n + T + 1]
+    gt = counts[2 * n + T + 1:]
+    pc, tpc = _above(by_class).t(), _above(hit).t()
+    P = torch.cat([(gt.sum() - pc.sum(1)).unsqueeze(1), pc], 1)
+    TP = torch.cat([(gt[0] - _above(bg_gt)).unsqueeze(1), tpc], 1)
+    return P, gt[:K].expand(T, K), TP
+
+
+class LabelEvaluator:
+    """evaluation.py's mIoU at every background threshold of a sweep, on the current CUDA device (csrc/label_eval.cu).
+
+    The result is exactly that of pseudo_label then label_iou run once per threshold: the counts are integers, and IoU and
+    mIoU are computed with label_iou's float64 formula.  thresholds: ascending floats (default i/100 for i in 0..99), compared
+    in float32 as pseudo_label compares them.  Counts accumulate over add / add_labels calls, so a dataset streams through in
+    batches; add_labels' label maps count the same at every threshold."""
+
+    def __init__(self, num_cls=21, thresholds=None):
+        self.num_cls = int(num_cls)
+        self.thresholds = [i / 100 for i in range(100)] if thresholds is None else [float(t) for t in thresholds]
+        self.device = torch.device("cuda", torch.cuda.current_device())
+        self._cam = torch.zeros(ops.cam_label_counts_len(self.num_cls, len(self.thresholds)), device=self.device, dtype=torch.int64)
+        self._map = torch.zeros(3, self.num_cls, device=self.device, dtype=torch.int64)
+
+    def add(self, cam_dicts, gt_maps):
+        """cam_dicts: {class: float [rows, cols]} per image (as load_cam_dict or infer_cam_batch return them); gt_maps: uint8
+        [rows, cols] per image (255 = ignore).  Images may differ in size.  One pinned buffer, one host-to-device copy."""
+        gt_maps = [np.asarray(g) for g in gt_maps]
+        assert len(cam_dicts) == len(gt_maps)
+        npix = [g.size for g in gt_maps]
+        nf = sum(len(d) * n for d, n in zip(cam_dicts, npix))
+        host = torch.empty(4 * nf + sum(npix), dtype=torch.uint8, pin_memory=True)
+        buf = host.numpy()
+        f, g = buf[:4 * nf].view(np.float32), buf[4 * nf:]
+        planes, images, fo, go = [], [], 0, 0
+        for m, (d, gt) in enumerate(zip(cam_dicts, gt_maps)):
+            assert gt.dtype == np.uint8 and gt.ndim == 2, "ground truth: uint8 [rows, cols]"
+            n = gt.size
+            g[go:go + n] = gt.reshape(-1)
+            images.append((go, gt.shape[0], gt.shape[1]))
+            go += n
+            for key, v in d.items():
+                assert np.shape(v) == gt.shape, f"image {m}: class {key} plane {np.shape(v)} vs ground truth {gt.shape}"
+                f[fo:fo + n] = np.asarray(v).reshape(-1)          # float32, as pseudo_label's tensor holds it
+                planes.append((fo, m, int(key)))
+                fo += n
+        dev = host.to(self.device, non_blocking=True)
+        ops.cam_label_counts(dev[:4 * nf].view(torch.float32), planes, dev[4 * nf:], images, self.thresholds, self.num_cls, self._cam)
+
+    def add_labels(self, pred_maps, gt_maps):
+        """Label-map predictions (uint8 [rows, cols], e.g. the argmax of crf_with_alpha's marginals) with their ground truth."""
+        pred_maps, gt_maps = [np.asarray(p) for p in pred_maps], [np.asarray(g) for g in gt_maps]
+        assert len(pred_maps) == len(gt_maps)
+        total = sum(g.size for g in gt_maps)
+        host = torch.empty(2 * total, dtype=torch.uint8, pin_memory=True)
+        buf = host.numpy()
+        images, o = [], 0
+        for p, gt in zip(pred_maps, gt_maps):
+            assert p.dtype == gt.dtype == np.uint8 and gt.ndim == 2 and p.shape == gt.shape, "label maps: uint8 [rows, cols]"
+            buf[o:o + gt.size] = p.reshape(-1)
+            buf[total + o:total + o + gt.size] = gt.reshape(-1)
+            images.append((o, gt.shape[0], gt.shape[1]))
+            o += gt.size
+        dev = host.to(self.device, non_blocking=True)
+        ops.label_map_counts(dev[:total], dev[total:], images, self.num_cls, self._map)
+
+    def counts(self):
+        """label_iou's P, T, TP at every threshold: int64 numpy [T, num_cls] each."""
+        P, T, TP = _curve_counts(self._cam, self.num_cls, len(self.thresholds))
+        return tuple((x + self._map[i]).cpu().numpy() for i, x in enumerate((P, T, TP)))
+
+    def result(self):
+        """(iou [T, num_cls] float64, miou [T] float64, best_threshold, best_miou): label_iou's values at every threshold; the
+        best threshold is the first one with the highest mIoU."""
+        P, T, TP = (x.astype(np.float64) for x in self.counts())
+        iou = TP / (T + P - TP + 1e-10)
+        miou = np.array([np.mean(r) for r in iou], dtype=np.float64)
+        best = int(np.argmax(miou))
+        return iou, miou, self.thresholds[best], float(miou[best])
+
+
+def label_iou_curve(cam_dicts, gt_maps, num_cls=21, thresholds=None):
+    """evaluation.py --curve in one call: LabelEvaluator(num_cls, thresholds), add, result."""
+    ev = LabelEvaluator(num_cls, thresholds)
+    ev.add(cam_dicts, gt_maps)
+    return ev.result()
+
+
 def _lowres_pass(model, both, present_idx, n_present, start_layer, getam_func, aff, t, normalize, max_replicas):
     """Device-only part of one scale of the batched path: trunk forward on both flips, blocks >= start_layer on one copy
     per present class, ONE backward, GETAM rows, affinity refinement.  Everything that depends on WHICH classes are present

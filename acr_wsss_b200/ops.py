@@ -764,6 +764,56 @@ def cam_finish(cams, patches, grids, labels, planes, total):
     return out
 
 
+def cam_label_counts_len(num_cls, num_thresholds):
+    """Length of the int64 counters of cam_label_counts: (2K-1)(T+1) + K + 1 for K = num_cls, T thresholds."""
+    return (2 * int(num_cls) - 1) * (int(num_thresholds) + 1) + int(num_cls) + 1
+
+
+def _table(rows, width):
+    t = np.ascontiguousarray(np.asarray(rows, dtype=np.int64).reshape(-1, width))
+    return t, t.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong))
+
+
+def cam_label_counts(cams, planes, gt, images, thresholds, num_cls, counts=None):
+    """Pseudo-label counts at every background threshold in one pass (csrc/label_eval.cu, acr_cam_label_counts).
+    cams: packed fp32 device buffer (for example ops.cam_finish's output); planes: host rows {offset, image, class} (dict class,
+    label class + 1); gt: packed uint8 device buffer; images: host rows {gt_offset, rows, cols}; thresholds: ascending floats.
+    Adds into `counts` (int64 device [cam_label_counts_len(num_cls, T)], zeros when None) and returns it; cam.LabelEvaluator
+    turns the counters into label_iou's P, T, TP per threshold."""
+    cams = torch.empty(0, device=gt.device, dtype=torch.float32) if cams is None else cams
+    _need_cuda(cams, gt)
+    assert cams.dtype == torch.float32 and cams.is_contiguous() and gt.dtype == torch.uint8 and gt.is_contiguous()
+    pl, pl_p = _table(planes, 3)
+    im, im_p = _table(images, 3)
+    th = np.ascontiguousarray(np.asarray(thresholds, dtype=np.float64).reshape(-1))
+    n = cam_label_counts_len(num_cls, len(th))
+    if counts is None:
+        counts = torch.zeros(n, device=gt.device, dtype=torch.int64)
+    assert counts.dtype == torch.int64 and counts.is_contiguous() and counts.numel() == n and counts.device == gt.device
+    wsb = _lib.lib().acr_label_counts_workspace(len(im), len(pl), len(th))
+    ws = torch.empty(max(wsb, 8), device=gt.device, dtype=torch.uint8)
+    _call("acr_cam_label_counts", 1 if len(im) else 0, _p(cams), cams.numel(), pl_p, len(pl), _p(gt), gt.numel(), im_p, len(im),
+          th.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), len(th), int(num_cls), _p(counts), _p(ws), wsb, _stream())
+    return counts
+
+
+def label_map_counts(pred, gt, images, num_cls, counts=None):
+    """label_iou's P, T, TP for label-map predictions (acr_label_map_counts): pred and gt packed uint8 device buffers of the same
+    length, images host rows {offset, rows, cols} (the same offset in both).  Adds into `counts` (int64 device [3, num_cls] =
+    P, T, TP; zeros when None) and returns it."""
+    _need_cuda(pred, gt)
+    assert pred.dtype == gt.dtype == torch.uint8 and pred.is_contiguous() and gt.is_contiguous() and pred.numel() == gt.numel()
+    im, im_p = _table(images, 3)
+    if counts is None:
+        counts = torch.zeros(3, int(num_cls), device=gt.device, dtype=torch.int64)
+    assert counts.dtype == torch.int64 and counts.is_contiguous() and counts.numel() == 3 * int(num_cls) and counts.device == gt.device
+    wsb = _lib.lib().acr_label_counts_workspace(len(im), 0, 0)
+    ws = torch.empty(max(wsb, 8), device=gt.device, dtype=torch.uint8)
+    _call("acr_label_map_counts", 1 if len(im) else 0, _p(pred), _p(gt), gt.numel(), im_p, len(im), int(num_cls), _p(counts),
+          _p(ws), wsb, _stream())
+    return counts
+
+
 class _PatchCam(torch.autograd.Function):
     """relu(tokens . W^T + b) through acr_patch_cam_tc; the backward (nobody on the reference path uses it: infer_cam.py:158
     detaches the result at once) is the plain closed form."""

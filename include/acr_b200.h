@@ -235,6 +235,45 @@ int acr_cam_finish(const float* const* cams_host, const float* const* patch_host
                    float* out, long long out_elems, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Pseudo-label evaluation.  Replaces evaluation.py:28-67 (pseudo_label's argmax over [tau, cam_1..cam_C], then label_iou's
+ * per-class P, T, TP) for a whole sweep of background thresholds in one pass, for a batch of images of any sizes.
+ * K = num_cls (1..255): labels 0 (background) .. K-1; a ground-truth pixel of 255 is ignored, one in [K, 255) is valid and
+ * matches no label (label_iou's `cal = gt < 255`).
+ *
+ * acr_cam_label_counts:
+ *   cams: packed fp32 planes (cam_elems floats); planes_host: HOST table of num_planes rows {offset, image, class}, the
+ *   rows*cols plane of dict class `class` (0..K-2, label class+1) of image `image` at cams + offset.  Planes may come in any
+ *   order; an image may have none; two planes of one image with the same class are rejected.
+ *   gt: packed uint8 ground truth (gt_elems bytes); images_host: HOST table of num_images rows {gt_offset, rows, cols},
+ *   1 <= rows*cols < 2^31.
+ *   thresholds_host: HOST array of T = num_thresholds (1..4096) doubles, finite and non-descending after float32 rounding
+ *   (equal neighbours are allowed); the comparison is made in float32, as pseudo_label's float32 tensor makes it.
+ *   Per pixel with gt != 255: (c*, m) = the FIRST maximum over labels 1..K-1 in label order, a label without a plane reading
+ *   0 (pseudo_label's zero planes; they decide when a threshold is negative or no plane is present); ties go to the lower
+ *   label whatever the table order; a NaN in any plane makes c* the first NaN label (np.argmax).  The pseudo-label at
+ *   threshold t is c* when m > float32(tau_t), else 0; j = #{t : float32(tau_t) < m} (a NaN m gives j = T).
+ *   counts: caller-owned int64 DEVICE counters, ADDED TO (so a dataset streams through in batches), Tp = T + 1:
+ *     [(K-1) * Tp] pixels with c* = c at row c-1, column j;   [(K-1) * Tp] the same with gt == c;
+ *     [Tp] pixels with gt == 0 by j;   [K + 1] pixels with gt == g (g < K), then valid pixels with gt >= K.
+ *   P, T, TP of label_iou at threshold t follow by suffix sums over j > t (cam.LabelEvaluator).
+ *   Envelope: histograms of (2K-1)*(T+1)*4 + 4K bytes <= 200 KB (COCO K = 81 up to T = 316, VOC K = 21 up to T = 1247).
+ *   workspace: >= acr_label_counts_workspace(num_images, num_planes, T) bytes, 8-byte aligned; receives the tables on
+ *   `stream`.  Deterministic (integer atomics).  No image launches nothing.
+ * acr_label_map_counts: label-map predictions (e.g. the argmax of crf_with_alpha's marginals).  pred and gt: packed uint8,
+ *   elems bytes each, image i at the same offset in both; images_host rows {offset, rows, cols}.  counts [3][K] int64 DEVICE,
+ *   added to: P[c] = #(pred == c), T[c] = #(gt == c), TP[c] = #(pred == gt == c) over pixels with gt != 255 (labels >= K count
+ *   in no class).  workspace: >= acr_label_counts_workspace(num_images, 0, 0) bytes, 8-byte aligned.
+ * Both reject null pointers, K out of range, a table row outside its buffer and a too-small workspace before any device work.
+ * ------------------------------------------------------------------------------------------ */
+size_t acr_label_counts_workspace(int num_images, int num_planes, int num_thresholds);
+int acr_cam_label_counts(const float* cams, long long cam_elems, const long long* planes_host, int num_planes,
+                         const unsigned char* gt, long long gt_elems, const long long* images_host, int num_images,
+                         const double* thresholds_host, int num_thresholds, int num_cls, long long* counts,
+                         void* workspace, size_t workspace_bytes, void* stream);
+int acr_label_map_counts(const unsigned char* pred, const unsigned char* gt, long long elems, const long long* images_host,
+                         int num_images, int num_cls, long long* counts, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Head of the dense-CRF regulariser (BASELINE configs[3]; call shape myTool.py:825-857, loop train_acr_coco.py:137-165):
  * the probabilities the bilateral filter sees, straight from the patch-token logits.
  *   logits [B,P*P,C] fp32 channel-last (cls_head(layer_4[:,1:]), DPT/ACR.py:133-134)
