@@ -3,8 +3,8 @@
 `infer_cam_image` reproduces the per-image loop body (scales x flips x present classes) with the hot pieces
 on this repo's kernels: head-mean stack (fused attention), GETAM from row-0 quantities, A = sum_l attn[:,l,1:,1:]
 and ONE [Np x Np]x[Np x C'] contraction for all present classes instead of C' matrix-vector products.
-Bilinear resizes are library calls (F.interpolate), exactly the ones the reference makes.  `infer_cam_batch` runs M images
-per trunk pass and finishes all of them (resizes to each image's own size, flips, sums, normalisation) in one kernel.
+`infer_cam_batch` runs M images per trunk pass; `infer_cam_image` is the same pass with M = 1.  Both finish every image
+(bilinear resizes to its own size, flips, sums over views and scales, min-max normalisation) in one kernel (ops.cam_finish).
 """
 import numbers
 import weakref
@@ -222,30 +222,12 @@ def label_iou_curve(cam_dicts, gt_maps, num_cls=21, thresholds=None):
     return ev.result()
 
 
-def _lowres_pass(model, both, present_idx, n_present, start_layer, getam_func, aff, t, normalize, max_replicas):
-    """Device-only part of one scale of the batched path: trunk forward on both flips, blocks >= start_layer on one copy
-    per present class, ONE backward, GETAM rows, affinity refinement.  Everything that depends on WHICH classes are present
-    goes through the device tensor `present_idx`, so the pass is CUDA-graph capturable per (shape, n_present).
-    Returns (patch_cam [2,Np,C], cams [2,Np,n_present])."""
-    rows_v = [[], []]
-    attn = patch_cam = None
-    for c0 in range(0, n_present, max_replicas):
-        n = min(max_replicas, n_present - c0)
-        cls_rep, _, attn, patch_cam = model.forward_cam_batched(both, n, start_layer)
-        model.backward_for_getam_batched(cls_rep, present_idx[c0:c0 + n].repeat(2))
-        for v in range(2):
-            for k in range(n):
-                cam, _, _ = model.getam(v * n + k, start_layer=start_layer, func=getam_func)
-                rows_v[v].append(cam[0])
-    cams = torch.stack([torch.stack(rows_v[v], dim=1) for v in range(2)])            # [2,Np,C']
-    if aff:
-        cams = torch.cat([affinity_refine(attn[v:v + 1].detach(), cams[v:v + 1], t=t, normalize=normalize) for v in range(2)])
-    return patch_cam.detach(), cams
-
-
-def _lowres_pass_batch(model, both, idx, n, start_layer, getam_func, aff, t, normalize):
-    """_lowres_pass for M images at once.  both [2M,3,h,w] (flipped views first), idx [2M*n] class of every (view, image, copy);
-    n copies per image (images with fewer present classes carry dummy copies).  Returns (patch_cam [2M,Np,C], cams [2M,Np,n])."""
+def _lowres_pass(model, both, idx, n, start_layer, getam_func, aff, t, normalize):
+    """Device-only part of one scale for M images: both [2M,3,h,w] (flipped views first) through the trunk, the blocks
+    >= start_layer on n copies of every sample, ONE backward, one batched GETAM, one affinity refinement.  idx [2M*n] is the
+    class of every (view, image, copy); images with fewer present classes carry dummy copies.  Which classes are present only
+    reaches the pass through that device tensor, so the pass is CUDA-graph capturable per (shape, n).
+    Returns (patch_cam [2M,Np,C], cams [2M,Np,n])."""
     cls_rep, _, attn, patch_cam = model.forward_cam_batched(both, n, start_layer)
     model.backward_for_getam_batched(cls_rep, idx)
     cams = model.getam_batch(start_layer=start_layer, func=getam_func)           # [2M*n, Np]
@@ -256,138 +238,63 @@ def _lowres_pass_batch(model, both, idx, n, start_layer, getam_func, aff, t, nor
 
 
 class _LowresGraph:
-    """CUDA graph of _lowres_pass for one (model, input shape, number of present classes, options) key: the pass is ~270
-    launches of small kernels at batch 2 and is CPU-launch bound when run eagerly (8.4 ms per image, 2.8 ms of GPU time).
+    """CUDA graph of _lowres_pass for one (model, input shape, copies per image, options) key: the pass is hundreds of
+    launches of small kernels and is CPU-launch bound when run eagerly.
     It lives in model._cam_graphs and holds the model weakly: a strong reference would make model and graphs cyclic garbage,
     and the cyclic collector could then destroy the graphs and free their memory pool in the middle of an unrelated CUDA graph
     capture, which invalidates that capture.  Without the cycle they go when the last reference to the model does."""
 
-    def __init__(self, model, shape, n_present, args, batch=False):
+    def __init__(self, model, shape, n, args):
         dev = next(model.parameters()).device
         self.both = torch.empty(shape, device=dev)
-        self.idx = torch.zeros(shape[0] * n_present if batch else n_present, device=dev, dtype=torch.long)
-        self.model, self.n, self.args = weakref.ref(model), n_present, args
-        self.fn = _lowres_pass_batch if batch else _lowres_pass
+        self.idx = torch.zeros(shape[0] * n, device=dev, dtype=torch.long)
+        self.model, self.n, self.args = weakref.ref(model), n, args
         self.graph = None
         self.calls = 0
         self.stream = torch.cuda.Stream(device=dev)
 
-    def run(self, both, present_idx):
+    def run(self, both, idx):
         self.both.copy_(both)
-        self.idx.copy_(present_idx)
+        self.idx.copy_(idx)
         self.calls += 1
         cur = torch.cuda.current_stream()
         if self.graph is None and self.calls <= 2:          # warm up eagerly on the capture stream (lazy inits, cuBLAS workspaces)
             self.stream.wait_stream(cur)
             with torch.cuda.stream(self.stream):
-                out = self.fn(self.model(), self.both, self.idx, self.n, *self.args)
+                out = _lowres_pass(self.model(), self.both, self.idx, self.n, *self.args)
             cur.wait_stream(self.stream)
             return out
         if self.graph is None:
             torch.cuda.synchronize()
             self.graph = torch.cuda.CUDAGraph()
             with ops.cuda_graph_capture(self.graph, self.stream):
-                self.out = self.fn(self.model(), self.both, self.idx, self.n, *self.args)
+                self.out = _lowres_pass(self.model(), self.both, self.idx, self.n, *self.args)
         self.graph.replay()
         return self.out
 
 
-def infer_cam_image(model, img, label, out_size, scales=(1,), start_layer=9, getam_func="cam_grad_s",
-                    aff=True, t=1, normalize=False, truncate_backward=True, batch_classes=True, max_replicas=8,
-                    cuda_graph=False):
-    """One image of the infer_cam.py loop body (:145-215).
+def infer_cam_image(model, img, label, out_size, scales=(1,), start_layer=9, getam_func="cam_grad_s", aff=True, t=1,
+                    normalize=False, cuda_graph=False):
+    """One image of the infer_cam.py loop body (:145-215): infer_cam_batch's pass and finish with M = 1.
 
     img [1,3,h,w] (normalised), label [1,C] multi-hot, out_size = (rows, cols) of the original image (the
-    reference calls these W,H at infer_cam.py:136).  Returns (cam_dict, patch_cam_dict, norm_cam [C,rows,cols])
-    with {class_index: float32 [rows,cols]} dicts as saved by np.save at :227-228.
-    truncate_backward: stop each per-class backward at block `start_layer` (identical GETAM; SURVEY section 8f rank 1).
-    batch_classes (needs truncate_backward): both flips go through the trunk as one batch of 2, the blocks >= start_layer
-    run on one copy of the token stream per present class (at most max_replicas per pass) and ONE backward delivers every
-    class's attention gradients for both flips.
-    cuda_graph (batched path on a GPU): replay the device-only part as a CUDA graph, cached on the model per (input shape,
+    reference calls these W,H at infer_cam.py:136).  Returns (cam_dict, patch_cam_dict, norm_cam): {class_index: float32
+    [rows,cols]} dicts as saved by np.save at :227-228 (views of one pinned host buffer), and the normalised GETAM maps on the
+    device, fp32 [C,rows,cols] with zeros for the absent classes.
+    cuda_graph (on a GPU): replay the device-only part as a CUDA graph, cached on the model per (input shape,
     number of present classes, options); the first two calls of a key run eagerly.  In-place weight updates are picked
     up by the replays (the graph reads the parameter storage); re-allocating parameters (e.g. model.to(...)) needs
     `model._cam_graphs.clear()`.
     """
     assert img.shape[0] == 1, "the reference infers one image at a time (infer_cam.py:122)"
-    C = label.shape[1]
-    b, c, h, w = img.shape
-    rows, cols = out_size
-    lab_host = label[0].tolist()                       # one device->host read (the reference tests the labels one by one)
-    present = [ci for ci in range(C) if lab_host[ci] > 1e-5]
-    cam_list, patch_cam_list = [], []
-    nblocks = len(model.pretrained.model.blocks)
-    batched = truncate_backward and batch_classes and len(present) > 0 and 0 < start_layer < nblocks
-    present_idx = torch.tensor(present, device=img.device, dtype=torch.long) if present else None
-
-    def finish_view(attn, patch_cam, cams, flipped, ph, pw):
-        """infer_cam.py:153-199 for one flip: patch CAM and (affinity-refined) GETAM maps at the original image size.
-        cams [1,Np,C'] (already refined when attn is None)."""
-        patch_cam = patch_cam.permute(0, 2, 1).reshape(1, C, ph, pw)
-        patch_cam = F.interpolate(patch_cam, [rows, cols], mode="bilinear", align_corners=False)[0]
-        patch_cam = patch_cam.detach() * label[0, :].view(C, 1, 1)
-        if flipped:
-            patch_cam = patch_cam.flip(-1)
-        patch_cam_list.append(patch_cam)
-        cam_matrix = torch.zeros(C, rows, cols, device=img.device)
-        if present:
-            if aff and attn is not None:
-                cams = affinity_refine(attn.detach(), cams, t=t, normalize=normalize)
-            cams = cams[0].t().reshape(len(present), 1, ph, pw)
-            cams = F.interpolate(cams, (rows, cols), mode="bilinear", align_corners=True)[:, 0]
-            cam_matrix.index_copy_(0, present_idx, cams)
-        if flipped:
-            cam_matrix = cam_matrix.flip(-1)
-        cam_list.append(cam_matrix)
-
-    for scale in scales:
-        inp = F.interpolate(img, size=(int(h * scale), int(w * scale)), mode="bilinear", align_corners=False)
-        ph, pw = int((h * scale) // 16), int((w * scale) // 16)
-        if batched:
-            # both flips as one batch of 2, every present class as a copy of the token stream from block start_layer on:
-            # one forward and ONE backward per scale (the reference: 2 forwards and 2*C' full backwards)
-            both = torch.cat([inp.flip(-1), inp], dim=0)          # hflip = 1 (flipped) first, then 2, as infer_cam.py:148-151
-            args = (start_layer, getam_func, aff, t, normalize, max_replicas)
-            if cuda_graph and img.is_cuda:
-                cache = model.__dict__.setdefault("_cam_graphs", {})
-                key = (tuple(both.shape), len(present)) + args
-                if key not in cache:
-                    if len(cache) >= 8:
-                        cache.clear()
-                    cache[key] = _LowresGraph(model, tuple(both.shape), len(present), args)
-                patch_cam, cams = cache[key].run(both, present_idx)
-            else:
-                patch_cam, cams = _lowres_pass(model, both, present_idx, len(present), *args)
-            for v in range(2):
-                finish_view(None, patch_cam[v:v + 1], cams[v:v + 1], v == 0, ph, pw)
-            continue
-        for hflip in (1, 2):
-            view = inp.flip(-1) if hflip % 2 == 1 else inp
-            cls_pred, _, attn, patch_cam = model.forward_cam(view)
-            output = cls_pred[0, :]
-            rows0 = []
-            for ci in present:
-                if truncate_backward:
-                    model.backward_for_getam(output[ci], start_layer)
-                else:
-                    # (set_to_none=False: a Trainer-attached model keeps its .grad views of the flat gradient buffer)
-                    model.zero_grad(set_to_none=False)
-                    output[ci].backward(retain_graph=True)      # one_hot * output, infer_cam.py:173-179
-                cam, _, _ = model.getam(0, start_layer=start_layer, func=getam_func)
-                rows0.append(cam[0])
-            cams = torch.stack(rows0, dim=1).unsqueeze(0) if present else None        # [1,Np,C']
-            finish_view(attn, patch_cam, cams, hflip % 2 == 1, ph, pw)
-    patch_sum = torch.stack(patch_cam_list).sum(0)
-    patch_norm = normalize_cam(patch_sum, 1e-5)
-    sum_cam = torch.stack(cam_list).sum(0)
-    norm_cam = normalize_cam(sum_cam, 1e-6)
-    # only the present classes go to the host (what the reference keeps, infer_cam.py:217-228), through one pinned buffer
-    if present:
-        both = torch.stack([norm_cam.index_select(0, present_idx), patch_norm.index_select(0, present_idx)])     # [2,C',rows,cols]
-        host_np = _to_host(both)
-    cam_dict = {ci: host_np[0, k] for k, ci in enumerate(present)}
-    patch_cam_dict = {ci: host_np[1, k] for k, ci in enumerate(present)}
-    return cam_dict, patch_cam_dict, norm_cam
+    rows, cols = int(out_size[0]), int(out_size[1])
+    out, _, (present,) = _infer_cams(model, img, label, [(rows, cols)], scales, start_layer, getam_func, aff, t, normalize,
+                                     cuda_graph)
+    k = len(present)
+    norm_cam = torch.zeros(label.shape[1], rows, cols, device=img.device)
+    norm_cam.index_copy_(0, torch.tensor(present, device=img.device, dtype=torch.long), out[:k * rows * cols].view(k, rows, cols))
+    host = _to_host(out).reshape(2, k, rows, cols)            # GETAM planes, then patch-CAM planes
+    return {ci: host[0, i] for i, ci in enumerate(present)}, {ci: host[1, i] for i, ci in enumerate(present)}, norm_cam
 
 
 def _to_host(t):
@@ -414,27 +321,13 @@ def _finish_planes(present, sizes):
     return planes, total
 
 
-def infer_cam_batch(model, imgs, labels, out_size, scales=(1,), start_layer=9, getam_func="cam_grad_s", aff=True, t=1,
-                    normalize=False, cuda_graph=False):
-    """infer_cam_image for M images of one input shape in ONE pass per scale (the reference loops over images,
-    infer_cam.py:122-215): both flips of all images go through the trunk as a batch of 2M, the blocks >= start_layer run on n
-    copies per image (n = the largest number of present classes in the batch; images with fewer classes carry dummy copies),
-    one backward, one batched GETAM, one batched affinity contraction.  Then ONE kernel (ops.cam_finish) resizes every
-    present class's GETAM map and patch CAM to its image's original size, adds the flips and scales and min-max normalises
-    them; dummy copies are never computed.
-    imgs [M,3,h,w] (the reference resizes every image to crop_size x crop_size first), labels [M,C]; out_size is the
-    original size (rows, cols) of every image, or a sequence of M such pairs when the originals differ.
-    Returns a list of (cam_dict, patch_cam_dict) per image, the same contents as infer_cam_image; the arrays are views of
-    one pinned host buffer.  An image without a present class gets two empty dicts."""
+def _infer_cams(model, imgs, labels, sizes, scales, start_layer, getam_func, aff, t, normalize, cuda_graph):
+    """infer_cam_batch on the device: sizes holds (rows, cols) per image.  Returns (ops.cam_finish's fp32 output buffer, its
+    plane table from _finish_planes, the present classes of every image)."""
     M, C = labels.shape
     assert imgs.shape[0] == M
-    if len(out_size) == 2 and all(isinstance(v, numbers.Integral) for v in out_size):
-        sizes = [(int(out_size[0]), int(out_size[1]))] * M
-    else:
-        sizes = [(int(r), int(c)) for r, c in out_size]
-        assert len(sizes) == M, "out_size: (rows, cols) or one such pair per image"
     nblocks = len(model.pretrained.model.blocks)
-    assert 0 < start_layer < nblocks, "the batched path stops the backward at block start_layer"
+    assert 0 <= start_layer < nblocks, "the backward stops at the input of block start_layer"
     lab_host = labels.tolist()                                   # one device->host read
     present = [[ci for ci in range(C) if lab_host[m][ci] > 1e-5] for m in range(M)]
     n = max(1, max(len(p) for p in present))
@@ -449,26 +342,49 @@ def infer_cam_batch(model, imgs, labels, out_size, scales=(1,), start_layer=9, g
         args = (start_layer, getam_func, aff, t, normalize)
         if cuda_graph and imgs.is_cuda:
             cache = model.__dict__.setdefault("_cam_graphs", {})
-            key = ("batch", tuple(both.shape), n) + args
+            key = (tuple(both.shape), n) + args
             if key not in cache:
                 if len(cache) >= 8:
                     cache.clear()
-                cache[key] = _LowresGraph(model, tuple(both.shape), n, args, batch=True)
+                cache[key] = _LowresGraph(model, tuple(both.shape), n, args)
             if key in live:            # a replay overwrites the graph's outputs: keep those of the earlier scale
                 j = live[key]
                 patch_s[j], cams_s[j] = patch_s[j].clone(), cams_s[j].clone()
             live[key] = len(cams_s)
             patch_cam, cams = cache[key].run(both, idx)
         else:
-            patch_cam, cams = _lowres_pass_batch(model, both, idx, n, *args)
+            patch_cam, cams = _lowres_pass(model, both, idx, n, *args)
         patch_s.append(patch_cam)
         cams_s.append(cams)
         grids.append((ph, pw))
     planes, total = _finish_planes(present, sizes)
-    host = _to_host(ops.cam_finish(cams_s, patch_s, grids, labels, planes, total))
+    return ops.cam_finish(cams_s, patch_s, grids, labels, planes, total), planes, present
+
+
+def infer_cam_batch(model, imgs, labels, out_size, scales=(1,), start_layer=9, getam_func="cam_grad_s", aff=True, t=1,
+                    normalize=False, cuda_graph=False):
+    """infer_cam_image for M images of one input shape in ONE pass per scale (the reference loops over images,
+    infer_cam.py:122-215): both flips of all images go through the trunk as a batch of 2M, the blocks >= start_layer run on n
+    copies per image (n = the largest number of present classes in the batch; images with fewer classes carry dummy copies),
+    one backward, one batched GETAM, one batched affinity contraction.  Then ONE kernel (ops.cam_finish) resizes every
+    present class's GETAM map and patch CAM to its image's original size, adds the flips and scales and min-max normalises
+    them; dummy copies are never computed.
+    imgs [M,3,h,w] (the reference resizes every image to crop_size x crop_size first), labels [M,C]; out_size is the
+    original size (rows, cols) of every image, or a sequence of M such pairs when the originals differ.
+    Returns a list of (cam_dict, patch_cam_dict) per image, the same contents as infer_cam_image; the arrays are views of
+    one pinned host buffer.  An image without a present class gets two empty dicts."""
+    M = labels.shape[0]
+    if len(out_size) == 2 and all(isinstance(v, numbers.Integral) for v in out_size):
+        sizes = [(int(out_size[0]), int(out_size[1]))] * M
+    else:
+        sizes = [(int(r), int(c)) for r, c in out_size]
+        assert len(sizes) == M, "out_size: (rows, cols) or one such pair per image"
+    out, planes, present = _infer_cams(model, imgs, labels, sizes, scales, start_layer, getam_func, aff, t, normalize,
+                                       cuda_graph)
+    host = _to_host(out)
     maps = iter(host[o:o + r * cl].reshape(r, cl) for o, _, _, _, r, cl in planes)
-    out = []
+    res = []
     for m in range(M):
         cam_dict = {ci: next(maps) for ci in present[m]}
-        out.append((cam_dict, {ci: next(maps) for ci in present[m]}))
-    return out
+        res.append((cam_dict, {ci: next(maps) for ci in present[m]}))
+    return res

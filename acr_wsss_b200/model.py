@@ -174,7 +174,7 @@ class Block(nn.Module):
     def forward_stream(self, x, pending, pending_bias=None, fold_out=True):
         """Same arithmetic as forward() with the residual adds folded into the LayerNorm kernels.  The residual stream
         travels as (x, pending) with the true value x + pending.  Returns (stream, pending branch, bias Parameter whose
-        gradient the NEXT add_layer_norm must produce (or None), this block's input)."""
+        gradient the NEXT add_layer_norm must produce (or None))."""
         if pending is None:
             s, h = x, self._norm(self.norm1, x)
         else:
@@ -184,7 +184,7 @@ class Block(nn.Module):
         s2, h2 = ops.add_layer_norm(s, self.attn(h, pb is not None), self.norm2.weight, self.norm2.bias, self.norm2.eps,
                                     out_bf16=True, branch_bias=pb)
         fb = _fold_bias(self.mlp.fc2, h2) if fold_out else None
-        return s2, self.mlp(h2, fb is not None), fb, s
+        return s2, self.mlp(h2, fb is not None), fb
 
 
 class PatchEmbed(nn.Module):
@@ -298,7 +298,6 @@ class VisionTransformer(nn.Module):
         cls_tokens = self.cls_token.expand(b, -1, -1)
         x = torch.cat((cls_tokens.to(x.dtype), x), dim=1)
         x = x + pos_embed.to(x.dtype)
-        self._block_in = []            # input of every block (references): lets GETAM stop its backward at start_layer
         self._rep_in = None
 
         def replicate(t):       # sample b -> copies b*replicas .. b*replicas + replicas - 1
@@ -318,14 +317,12 @@ class VisionTransformer(nn.Module):
                 if i == replicate_at:
                     assert pbias is None, "batched GETAM runs outside the training path"
                     x, pending = replicate(x if pending is None else x + pending), None
-                x, pending, pbias, blk_in = blk.forward_stream(x, pending, pbias, fold_out=i + 1 < len(self.blocks))
-                self._block_in.append(blk_in)
+                x, pending, pbias = blk.forward_stream(x, pending, pbias, fold_out=i + 1 < len(self.blocks))
             x = x + pending
         else:
             for i, blk in enumerate(self.blocks):
                 if i == replicate_at:
                     x = replicate(x)
-                self._block_in.append(x)
                 x = blk(x)
         if last_block_out is not None:
             last_block_out.append(x)
@@ -528,12 +525,6 @@ class ACR(nn.Module):
         p0 = torch.stack([blk.attn.get_attn_row0() for blk in used])               # [L',S,H,N]
         g0 = torch.stack([blk.attn.get_attn_gradients_row0() for blk in used])
         return ops.getam_row0_batch(p0, g0, 0, func, skip)
-
-    def backward_for_getam(self, logit, start_layer=0):
-        """Gradient pass that feeds getam().  The reference calls logit.backward(retain_graph=True) through the whole
-        model and all parameters (infer_cam.py:173-179); only dP of blocks >= start_layer is ever read, so this stops
-        at the input of block `start_layer` and accumulates no parameter gradients (same GETAM result)."""
-        torch.autograd.grad(logit, self.pretrained.model._block_in[start_layer], retain_graph=True)
 
 
 def _getam_full(cam, grad, func):

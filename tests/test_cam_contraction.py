@@ -320,9 +320,9 @@ def _lowres_bytes(grids):
 
 
 def _reference_finish(cams_s, patch_s, grids, labels, present, sizes):
-    """infer_cam_image's finish as torch ops, for any grid set (non-square grids included): per image (GETAM planes
-    [n_m,rows,cols], patch-CAM planes [n_m,rows,cols]) summed over scales, then views (view 0 = flipped input, first), then
-    min-max normalised."""
+    """The reference's finish (infer_cam.py:153-215) as torch ops, for any grid set (non-square grids included): per image
+    (GETAM planes [n_m,rows,cols], patch-CAM planes [n_m,rows,cols]) summed over scales, then views (view 0 = flipped input,
+    first), then min-max normalised."""
     from acr_wsss_b200.cam import normalize_cam
     M, C = labels.shape
     out = []

@@ -1,6 +1,6 @@
 """GPU tier (-m gpu): batched CAM inference for images of different original sizes.
 
-The finish kernel (ops.cam_finish, csrc/cam_finish.cu) against the torch composition of infer_cam_image's finish, and
+The finish kernel (ops.cam_finish, csrc/cam_finish.cu) against the reference's finish as torch ops, and
 infer_cam_batch with per-image output sizes against infer_cam_image run image by image.
 """
 import numpy as np
@@ -30,8 +30,9 @@ def _build(dev, C, precision, qkv_gain=2.0):
 
 
 def _reference_finish(cams_s, patch_s, grids, labels, present, sizes):
-    """infer_cam_image's finish (cam.py finish_view, the stacked sums and normalize_cam) for each image of the batch:
-    returns per image (GETAM planes [n_m,rows,cols], patch-CAM planes [n_m,rows,cols])."""
+    """The reference's finish (infer_cam.py:153-215: F.interpolate per view, label multiply, flip, sums over views and
+    scales, normalize_cam) as torch ops for each image of the batch: returns per image (GETAM planes [n_m,rows,cols],
+    patch-CAM planes [n_m,rows,cols])."""
     from acr_wsss_b200.cam import normalize_cam
     M, C = labels.shape
     out = []

@@ -318,7 +318,7 @@ def test_patch_cam_tc(dev, B, M, E, C, rep):
     assert rel_err(t2n(td.grad), gx.numpy()) < 1e-4
 
 
-def _infer_check(dev, name, precision, tol, truncate=True, batch_classes=True):
+def _infer_check(dev, name, precision, tol):
     from acr_wsss_b200 import infer_cam_image, pseudo_label, synth
     g = load_golden(name)
     C, S = int(g["C"]), int(g["S"])
@@ -329,8 +329,7 @@ def _infer_check(dev, name, precision, tol, truncate=True, batch_classes=True):
     label = synth.labels(1, C, present=present).to(dev)
     cam_dict, patch_dict, norm_cam = infer_cam_image(m, img, label, tuple(int(v) for v in g["out_size"]),
                                                      scales=tuple(float(s) for s in g["scales"]),
-                                                     start_layer=int(g["start_layer"]), getam_func=str(g["func"]),
-                                                     truncate_backward=truncate, batch_classes=batch_classes)
+                                                     start_layer=int(g["start_layer"]), getam_func=str(g["func"]))
     assert sorted(cam_dict) == present and cam_dict[present[0]].dtype == np.float32
     assert rel_err(np.stack([cam_dict[c] for c in present]), g["norm_cam"]) < tol
     assert rel_err(np.stack([patch_dict[c] for c in present]), g["patch_norm_cam"]) < tol
@@ -366,13 +365,26 @@ def test_infer_cam_fp32_multiscale(dev):
     _infer_check(dev, "infer_vitb_128_ms.npz", "fp32", FP32_TOL)
 
 
-def test_infer_cam_fp32_per_class_truncated_backward(dev):
-    """One truncated backward per class (the batched-GETAM default is covered by the tests above)."""
-    _infer_check(dev, "infer_vitb_128_ms.npz", "fp32", FP32_TOL, batch_classes=False)
-
-
-def test_infer_cam_fp32_multiscale_full_backward(dev):
-    _infer_check(dev, "infer_vitb_128_ms.npz", "fp32", FP32_TOL, truncate=False)
+def test_infer_cam_fp32_start_layer_0(dev):
+    """start_layer = 0: the class copies start at the input of block 0 (forward_flex(replicate_at=0)) and GETAM sums over
+    every block; against the oracle's loop (one full backward per class) run on the same weights and inputs."""
+    from acr_wsss_b200 import infer_cam_image, pseudo_label, synth
+    orc = _orc()
+    C, present, out_size = 20, [2, 9, 14], (40, 36)
+    m, sd = _build(dev, C, "vitb", "fp32")
+    m.eval()
+    img = synth.images(1, 128, seed=3)
+    label = synth.labels(1, C, present=present)
+    kw = dict(scales=(1.0, 0.5), start_layer=0, getam_func="cam_grad_s")
+    cam_dict, patch_dict, norm_cam = infer_cam_image(m, img.to(dev), label.to(dev), out_size, **kw)
+    ref_cam, ref_patch, ref_norm = orc.infer_cam_image(sd, img, label, out_size, **kw)
+    assert sorted(cam_dict) == present and sorted(patch_dict) == present
+    assert rel_err(np.stack([cam_dict[c] for c in present]), np.stack([ref_cam[c] for c in present])) < FP32_TOL
+    assert rel_err(np.stack([patch_dict[c] for c in present]), np.stack([ref_patch[c] for c in present])) < FP32_TOL
+    assert rel_err(t2n(norm_cam), ref_norm) < FP32_TOL
+    for t in (0.25, 0.40):
+        agree = (pseudo_label(cam_dict, C, t) == orc.pseudo_label(ref_cam, C, t)).mean()
+        assert agree >= 0.999, (t, agree)
 
 
 def test_infer_cam_batch_matches_per_image(dev):
