@@ -66,6 +66,12 @@ SIGNATURES = {
     "acr_pamr_workspace": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int]),
     "acr_pamr_fwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                              POINTER(c_int), c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "acr_pamr_save_workspace": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int, c_int]),
+    "acr_pamr_fwd_save": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                  POINTER(c_int), c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "acr_pamr_bwd_workspace": (c_size_t, [c_int, c_int, c_int, c_int, c_int, c_int]),
+    "acr_pamr_bwd": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                             POINTER(c_int), c_int, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "acr_bilateral_workspace": (c_size_t, [c_int, c_int, c_int, c_int]),
     "acr_bilateral_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_float,
                                     c_void_p, c_size_t, POINTER(c_int), c_void_p]),

@@ -884,12 +884,53 @@ def crf_head(logits, S):
 # ----------------------------------------------------------------------------------------------
 # (a10) PAMR, (a11) bilateral
 # ----------------------------------------------------------------------------------------------
+class _Pamr(torch.autograd.Function):
+    """PAMR with gradients to the mask and the image: the forward keeps the weights and the iterates M_0..M_{T-1}
+    (acr_pamr_fwd_save, output bitwise equal to acr_pamr_fwd's), the backward runs only the kernels the requested
+    gradients need (acr_pamr_bwd; with the mask alone, none of the image-side ones)."""
+
+    @staticmethod
+    def forward(ctx, x, mask, dilations, num_iter):
+        B, K, H, W = x.shape
+        _, C, mh, mw = mask.shape
+        nd = len(dilations)
+        dil = (ctypes.c_int * nd)(*dilations)
+        out = torch.empty(B, C, H, W, device=x.device, dtype=torch.float32)
+        sb = _lib.lib().acr_pamr_save_workspace(B, K, C, H, W, nd, num_iter)
+        saved = torch.empty(sb, device=x.device, dtype=torch.uint8)
+        _call("acr_pamr_fwd_save", 3, _p(x), _p(mask), B, K, C, H, W, mh, mw, dil, nd, num_iter, _p(out), _p(saved), sb, _stream())
+        ctx.save_for_backward(x, saved)
+        ctx.dims = (B, K, C, H, W, mh, mw, dilations, num_iter)
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g_out):
+        x, saved = ctx.saved_tensors
+        B, K, C, H, W, mh, mw, dilations, num_iter = ctx.dims
+        need_x, need_mask = ctx.needs_input_grad[:2]
+        d_x = torch.empty_like(x) if need_x else None
+        d_mask = torch.empty(B, C, mh, mw, device=x.device, dtype=torch.float32) if need_mask else None
+        nd = len(dilations)
+        wsb = _lib.lib().acr_pamr_bwd_workspace(B, K, C, H, W, nd)
+        ws = torch.empty(wsb, device=x.device, dtype=torch.uint8)
+        g_out = g_out.contiguous().float()
+        adjoints = num_iter - 1 + int(need_mask) if num_iter > 0 else 0
+        nlaunch = adjoints + int(need_mask) + (num_iter + 2 if need_x else 0)
+        _call("acr_pamr_bwd", nlaunch, _p(x), _p(saved), saved.numel(), _p(g_out), B, K, C, H, W, mh, mw,
+              (ctypes.c_int * nd)(*dilations), nd, num_iter, _p(d_x), _p(d_mask), _p(ws), wsb, _stream())
+        return d_x, d_mask, None, None
+
+
 def pamr_forward(x, mask, dilations, num_iter):
     _need_cuda(x, mask)
     B, K, H, W = x.shape
     _, C, mh, mw = mask.shape
     x = x.contiguous().float()
     mask = mask.contiguous().float()
+    if torch.is_grad_enabled() and (x.requires_grad or mask.requires_grad):
+        # with no iteration the output is the up-sampled mask alone: x is not part of the graph, as in the reference
+        return _Pamr.apply(x if num_iter > 0 else x.detach(), mask, [int(d) for d in dilations], int(num_iter))
     nd = len(dilations)
     dil = (ctypes.c_int * nd)(*[int(d) for d in dilations])
     out = torch.empty(B, C, H, W, device=x.device, dtype=torch.float32)

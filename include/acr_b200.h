@@ -298,6 +298,24 @@ size_t acr_pamr_workspace(int B, int K, int C, int H, int W, int nd);
 int acr_pamr_fwd(const float* x, const float* mask, int B, int K, int C, int H, int W, int mh, int mw,
                  const int* dilations_host, int nd, int num_iter,
                  float* out, void* workspace, size_t workspace_bytes, void* stream);
+/* Backward of PAMR.forward with respect to the mask and the image (first order, fp32).
+ * acr_pamr_fwd_save: the forward with its state kept for the backward.  out is bitwise equal to acr_pamr_fwd's.  saved:
+ *   caller-owned, acr_pamr_save_workspace() bytes (the affinity weights and the num_iter padded iterates M_0 .. M_{T-1}),
+ *   256-byte aligned; it must stay untouched until acr_pamr_bwd has run.
+ * acr_pamr_bwd: g_out [B,C,H,W] = dL/dout -> d_mask [B,C,mh,mw] and d_x [B,K,H,W] (either may be NULL, not both; with
+ *   d_x NULL the image-side kernels do not run; num_iter = 0 writes d_x as zeros).  Same shapes, dilations and num_iter as
+ *   the acr_pamr_fwd_save call that filled `saved`.  workspace: acr_pamr_bwd_workspace() bytes, 256-byte aligned.
+ *   Deterministic (gathers, no atomics); no host synchronisation and no allocation, so it can be captured in a CUDA graph.
+ * Both reject null pointers, shapes <= 0, nd outside 1..8, a dilation < 1, num_iter < 0, short buffers and grids beyond
+ * H <= 65535, B*C <= 65535 before any device work. */
+size_t acr_pamr_save_workspace(int B, int K, int C, int H, int W, int nd, int num_iter);
+int acr_pamr_fwd_save(const float* x, const float* mask, int B, int K, int C, int H, int W, int mh, int mw,
+                      const int* dilations_host, int nd, int num_iter,
+                      float* out, void* saved, size_t saved_bytes, void* stream);
+size_t acr_pamr_bwd_workspace(int B, int K, int C, int H, int W, int nd);
+int acr_pamr_bwd(const float* x, const void* saved, size_t saved_bytes, const float* g_out, int B, int K, int C, int H, int W,
+                 int mh, int mw, const int* dilations_host, int nd, int num_iter, float* d_x, float* d_mask,
+                 void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * (a11) Permutohedral bilateral filter.  Replaces bilateralfilter_batch,
